@@ -2,7 +2,7 @@
 """bench.py -- MPC solves/s on the BASELINE.json workloads.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
-                  [--workload batch64k|weights1M|grid256k|rollout8192x1000]
+                  [--workload batch64k|weights1M|grid256k|rollout8192x1000] [--dump-outputs DIR]
 
 Default workload (the metric BASELINE.json is quoted on, configs[1]): a "step" is one pass of the hot path (one
 `mpc_solve_batch` launch chain) over one batch of B = 65 536 synthetic problems per GPU -- perturbed poses along
@@ -407,6 +407,29 @@ def status_hist(st):
     return {str(int(k)): int(v) for k, v in zip(u, c)}
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each array as out_dir/<name>.npy in float64 (status and iteration counts are exact there).
+    The last axis of every array indexes the problem (or vehicle).  When all of them together would pass DUMP_MAX_BYTES,
+    every array keeps the same fixed, seeded sample of problems, whose indices go to sample_index.npy."""
+    arrays = {k: np.asarray(v.cpu().numpy() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[-1]
+    assert all(a.shape[-1] == n for a in arrays.values()), {k: a.shape for k, a in arrays.items()}
+    per_problem = 8 * sum(a.size // max(n, 1) for a in arrays.values())
+    room = DUMP_MAX_BYTES - 128 * (len(arrays) + 1)          # an .npy header is 128 bytes
+    if per_problem * n > room:
+        keep = room // (per_problem + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[..., idx] for k, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
+    log("outputs of the last timed step written to %s: %s" % (out_dir, ", ".join(sorted(arrays))))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # BASELINE configs[2..4] as written, sharded over the ranks
 # ---------------------------------------------------------------------------------------------------------------
@@ -434,6 +457,8 @@ def run_weights1M(ctx, args):
     S = mpc.Solver(cfg, ctx.local_rank)
     step = lambda k: S.solve_batch_device(B, *ins, res, None, None, None, st, it, weights=Wd)
     ms, _ = timed_steps(ctx, step, args.steps, max(3, args.warmup))
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, {"result": res, "status": st, "iters": it})
     ms_step = ctx.max_over_ranks(sum(ms)) / args.steps
     iters_sum = ctx.sum_over_ranks(float(it.sum().item()))
     ok = ctx.sum_over_ranks(float((st == 1).sum().item())) / Btot
@@ -473,6 +498,8 @@ def run_grid256k(ctx, args):
     st = torch.zeros(B, dtype=torch.int32, device=ctx.dev); it = torch.zeros(B, dtype=torch.int32, device=ctx.dev)
     step = lambda k: S.solve_batch_device(B, *ins, res, None, None, None, st, it, N_per=Np, dt_per=dtp)
     ms, _ = timed_steps(ctx, step, args.steps, max(3, args.warmup))
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, {"result": res, "status": st, "iters": it})
     ms_step = ctx.max_over_ranks(sum(ms)) / args.steps
     stn, itn = st.cpu().numpy(), it.cpu().numpy()
     flops = float(sum(f_iter(n) * itn[Nall[lo:hi] == n].sum() for n in (10, 20, 30, 40, 50)))
@@ -522,16 +549,18 @@ def run_rollout(ctx, args):
         S.rollout_device(V, T, wx, wy, state["veh"], state["seg"], state["pend"], 0.1, 0.02, rec)
 
     n0 = S.launches
-    ms, _ = timed_steps(ctx, step, max(1, args.steps), 1)
-    launches = (S.launches - n0) // (max(1, args.steps) + 1)
-    ms_roll = ctx.max_over_ranks(sum(ms)) / max(1, args.steps)
+    ms, _ = timed_steps(ctx, step, args.steps, 1)
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, {"rec": rec, "veh": state["veh"], "seg": state["seg"], "pending": state["pend"]})
+    launches = (S.launches - n0) // (args.steps + 1)
+    ms_roll = ctx.max_over_ranks(sum(ms)) / args.steps
     r = rec.cpu().numpy()
     ok = ctx.sum_over_ranks(float((r[:, 6] == 1).sum())) / (Vtot * T)
     iters_sum = ctx.sum_over_ranks(float(r[:, 7].sum()))
     fp64 = mpc.measure_fp64_peak(ctx.local_rank)
     tf = f_iter(cfg.N) * iters_sum / (ms_roll * 1e-3) / 1e12
     line = {"metric": "closed-loop vehicle-steps/sec (8192 vehicles x 1000 steps, config-fast, 100 ms latency)", "value": Vtot * T / (ms_roll * 1e-3),
-            "unit": "vehicle-steps/s", "n_gpus": ctx.world, "steps": max(1, args.steps), "warmup": 1, "ms_per_step": ms_roll, "higher_is_better": True,
+            "unit": "vehicle-steps/s", "n_gpus": ctx.world, "steps": args.steps, "warmup": 1, "ms_per_step": ms_roll, "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": {"workload": "configs[4]: 100 ms latency-compensated closed-loop rollouts, %d vehicles x %d control steps of 0.1 s (config-fast, tau_solve 0.02 s), "
                                    "vehicles sharded over %d rank(s); a 'step' of this line is one whole rollout" % (Vtot, T, ctx.world),
@@ -640,6 +669,8 @@ def run_batch64k(ctx, args):
     it = si[jl][1].cpu().numpy()
     st = si[jl][0].cpu().numpy()
     res_last = result[jl]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"result": res_last, "traj_x": tx, "traj_y": ty, "status": st, "iters": it})
     flops_per_launch = float(f_iter(N)) * float(it.sum())
     kernel_ms = float(np.mean(step_ms))      # the launches of one solve on this rank
 
@@ -930,7 +961,15 @@ def main():
     ap.add_argument("--gather", default="serial", choices=["overlap", "serial"],
                     help="multi-GPU: the gather of step k finishes before the solve of step k+1 starts (default), or runs beside it (see DESIGN.md section 7)")
     ap.add_argument("--only-timed", action="store_true", help="development: the timed region only (no strong-scaling, host-API, latency, extras or CPU legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's arrays, [k][B] layout as the caller "
+                         "receives them) as DIR/<name>.npy in float64, at most 64 MB in all: a fixed, seeded sample of the "
+                         "problems beyond that.  The inputs depend only on the arguments, so two builds can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours (the reference arm times a sample sized by its own speed)")
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank)

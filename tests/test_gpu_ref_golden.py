@@ -132,11 +132,12 @@ def test_cpp_host_class_runs_testcpp_scenario(gold, refdata, tmp_path):
 
 def test_dropin_mpc_cpp_in_reference_tree(gold, refdata, tmp_path):
     """oracle/_ref/dropin_testcpp = the reference's Vehicle/RoadGeometry/utils/Config sources + OUR
-    src/control/MPC.cpp (integration/reference_tree) + a driver making test.cpp's calls; built in the
-    build container (needs /root/reference), run here on the GPU."""
+    src/control/MPC.cpp (integration/reference_tree) + a driver making test.cpp's calls; built by
+    `make -C oracle/ref_shim REF=<checkout of the original project>` (those sources are not part of this
+    repository), run here on the GPU."""
     exe = os.path.join(ROOT, "oracle", "_ref", "dropin_testcpp")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/dropin_testcpp not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/dropin_testcpp not built (needs the original project's sources: make -C oracle/ref_shim REF=...)")
     for fx, sc in zip(refdata["test_cpp_fixtures"][:2], gold["testcpp"][:2]):
         out = subprocess.run([exe] + _scenario_args(refdata, fx, tmp_path), capture_output=True, text=True, timeout=300)
         assert out.returncode == 0, out.stderr

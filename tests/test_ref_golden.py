@@ -112,11 +112,12 @@ def test_host_run_logic_errors(mpc, stable_cfg):
 
 
 def test_live_reference_build_agrees_with_oracle(po, refdata):
-    """Where oracle/_ref exists (it is built from /root/reference in the build container and travels with
-    the snapshot), run the reference's code live: Config::load and fresh random problems."""
+    """Where oracle/_ref exists (built by `make -C oracle/ref_shim REF=<checkout of the original project>`; the
+    original project's sources are not part of this repository), run the reference's code live: Config::load and
+    fresh random problems."""
     from oracle import pyref as pr
     if not pr.available():
-        pytest.skip("oracle/_ref/libmpc_ref.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libmpc_ref.so not built (needs the original project's sources: make -C oracle/ref_shim REF=...)")
     import mpc_b200 as mpc
     for name in ("stable", "fast", "no-latency"):
         js = refdata["configs"][name]
