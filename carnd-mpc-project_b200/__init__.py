@@ -35,7 +35,8 @@ EXPORTS = ["mpc_config_defaults", "mpc_config_load_json", "mpc_config_parse_json
            "mpc_run_prepare", "mpc_run_finish", "mpc_compute_throttle", "mpc_vehicle_move", "mpc_run_batch",
            "mpc_rollout", "mpc_set_handoff", "mpc_set_tail", "mpc_tail_counts", "mpc_measure_solve_latency", "mpc_set_dual_outputs", "mpc_config_from_cli",
            "mpc_telemetry_parse", "mpc_telemetry_step", "mpc_create_multi", "mpc_destroy_multi", "mpc_multi_device_count",
-           "mpc_multi_handle", "mpc_solve_batch_multi", "mpc_set_rollout_mode"]
+           "mpc_multi_handle", "mpc_solve_batch_multi", "mpc_set_rollout_mode", "mpc_set_warm_start", "mpc_warm_start_shift",
+           "mpc_set_warm_start_one"]
 
 
 class MpcError(RuntimeError):
@@ -125,6 +126,9 @@ def lib():
     L.mpc_tail_counts.argtypes = [vp, C.POINTER(C.c_int), C.c_int]
     L.mpc_measure_solve_latency.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.mpc_set_dual_outputs.argtypes = [vp, vp, vp, vp]
+    L.mpc_set_warm_start.argtypes = [vp, vp, vp, vp, vp, C.c_double]
+    L.mpc_set_warm_start_one.argtypes = [vp, C.c_int, C.c_double]
+    L.mpc_warm_start_shift.argtypes = [vp, C.c_int] + [vp] * 8 + [vp]
     L.mpc_telemetry_parse.argtypes = [C.c_char_p, C.POINTER(MpcTelemetry)]
     L.mpc_telemetry_step.argtypes = [vp, C.c_char_p, dp, C.c_double, C.c_int, C.c_char_p, C.c_int]
     L.mpc_solve_batch.argtypes = [vp, C.c_int] + [vp] * 13 + [vp]
@@ -188,6 +192,15 @@ class MultiSolver:
         _check(lib().mpc_solve_batch_multi(self._m, B, _ptr(state), _ptr(coeffs), _ptr(yaw_lo), _ptr(yaw_hi), _ptr(weights),
                                            _ptr(N_per), _ptr(dt_per), _ptr(result), _ptr(traj_x), _ptr(traj_y), _ptr(full),
                                            _ptr(status), _ptr(iters)), "mpc_solve_batch_multi")
+
+    def set_warm_start(self, g, x0=None, lam0=None, zl0=None, zu0=None, mu_init=0.0):
+        """Warm start of shard g (problems [g*B/G, (g+1)*B/G)): device tensors on that shard's device, see
+        Solver.set_warm_start."""
+        self._warm = getattr(self, "_warm", {})
+        self._warm[g] = (x0, lam0, zl0, zu0)   # keep them alive
+        h = lib().mpc_multi_handle(self._m, int(g))
+        _check(lib().mpc_set_warm_start(h, _ptr(x0), _ptr(lam0), _ptr(zl0), _ptr(zu0), float(mu_init)),
+               "mpc_set_warm_start")
 
     def solve_batch_host(self, state, coeffs, yaw_lo, yaw_hi, weights=None, N_per=None, dt_per=None, want_full=False):
         B, N = state.shape[0], self.cfg.N
@@ -360,6 +373,26 @@ class Solver:
         """Device tensors lam [6N][B], zl, zu [8N-2][B] receiving the multipliers of later solves (None = off)."""
         self._dual = (lam, zl, zu)   # keep them alive
         _check(lib().mpc_set_dual_outputs(self._h, _ptr(lam), _ptr(zl), _ptr(zu)), "mpc_set_dual_outputs")
+
+    def set_warm_start(self, x0=None, lam0=None, zl0=None, zu0=None, mu_init=0.0):
+        """Warm start of later batch solves (mpc_set_warm_start): device tensors x0 [8N-2][B] (as ``full``), lam0 [6N][B],
+        zl0, zu0 [8N-2][B] (as the dual outputs; each may be None), unscaled; mu_init 0 = Ipopt's 0.1.  x0 None = off."""
+        self._warm = (x0, lam0, zl0, zu0)   # keep them alive
+        _check(lib().mpc_set_warm_start(self._h, _ptr(x0), _ptr(lam0), _ptr(zl0), _ptr(zu0), float(mu_init)),
+               "mpc_set_warm_start")
+
+    def set_warm_start_one(self, on, mu_init=0.0):
+        """solve_one starts from its previous solution shifted by one stage (mpc_set_warm_start_one)."""
+        _check(lib().mpc_set_warm_start_one(self._h, int(bool(on)), float(mu_init)), "mpc_set_warm_start_one")
+
+    def warm_start_shift(self, B, x, x0, lam=None, lam0=None, zl=None, zl0=None, zu=None, zu0=None, stream=None):
+        """Receding-horizon shift of a solution into the next step's start point (mpc_warm_start_shift), device
+        tensors in the layouts of set_warm_start; asynchronous on ``stream`` (None = torch's current stream)."""
+        if stream is None:
+            import torch
+            stream = torch.cuda.current_stream().cuda_stream
+        _check(lib().mpc_warm_start_shift(self._h, int(B), _ptr(x), _ptr(lam), _ptr(zl), _ptr(zu), _ptr(x0), _ptr(lam0),
+                                          _ptr(zl0), _ptr(zu0), stream), "mpc_warm_start_shift")
 
     @property
     def launches(self):

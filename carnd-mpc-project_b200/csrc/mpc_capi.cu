@@ -75,6 +75,13 @@ struct mpc_handle {
   int *d_perm;          // ragged batches: problem order of the work queue (longest horizon first)
   size_t cap_perm;
   double *dual_lam, *dual_zl, *dual_zu;   // caller's device buffers for the multipliers (or NULL)
+  const double *ws_x, *ws_lam, *ws_zl, *ws_zu;   // caller's device buffers of a warm start (ws_x NULL: cold start)
+  double ws_mu;                                  // its initial barrier parameter
+  // mpc_set_warm_start_one: mpc_solve_one keeps its last solution (x, lambda, zl, zu) in d_one and starts from it shifted
+  bool one_warm, one_prev_ok;
+  double one_mu;
+  double *d_one;        // [2][x 8N-2 | lambda 6N | zl 8N-2 | zu 8N-2]: the last solution, the next start point
+  int one_N;
   // staging buffers for the host-pointer entry points (grown on demand)
   double *d_in, *d_out;
   int *d_iout;
@@ -364,6 +371,7 @@ extern "C" void mpc_destroy(mpc_handle *h) {
   cudaFreeHost(h->h_pin);
   cudaFree(h->d_run);
   cudaFree(h->d_run_i);
+  cudaFree(h->d_one);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream2) cudaStreamDestroy(h->stream2);
   if (h->ev_pre) cudaEventDestroy(h->ev_pre);
@@ -376,6 +384,7 @@ extern "C" int mpc_set_config(mpc_handle *h, const mpc_config *cfg) {
   int rc = check_config(cfg);
   if (rc) return rc;
   h->cfg = *cfg;
+  h->one_prev_ok = false;   // a solution of another problem definition is no start point
   return MPC_OK;
 }
 
@@ -447,35 +456,35 @@ static int ensure_restart(mpc_handle *h, KParams &kp) {
 #define MPC_LANE_MINB 1   // CTAs per SM the lane kernel is compiled for (__launch_bounds__(256, MINB)): experiments only
 #endif
 // the final launch of a lane-kernel chain: the coop kernel on the parked / handed-over records and the restart list
-template <int NS>
+template <int NS, bool WARM>
 static int launch_finisher(mpc_handle *h, KParams &kp, cudaStream_t st, long long max_work) {
   const int ct = 128, G = NS <= 16 ? 16 : 32, groups = ct / G;
   const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
   static thread_local int cached_dev2 = -1;
   if (cached_dev2 != h->device) {
-    CK(cudaFuncSetAttribute(mpc_coop_resume_kernel<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(cudaFuncSetAttribute(mpc_coop_resume_kernel<NS, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cached_dev2 = h->device;
   }
   int per_sm = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_resume_kernel<NS>, ct, smem));
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_resume_kernel<NS, WARM>, ct, smem));
   if (per_sm < 1) per_sm = 1;
   long long g2 = (long long)h->sm_count * per_sm, w2 = (max_work + groups - 1) / groups;
   if (g2 > w2) g2 = w2;
   if (g2 < 1) g2 = 1;
   int rc = ensure_coop_scratch<NS>(h, kp, g2 * groups);
   if (rc) return rc;
-  mpc_coop_resume_kernel<NS><<<(unsigned)g2, ct, smem, st>>>(kp);
+  mpc_coop_resume_kernel<NS, WARM><<<(unsigned)g2, ct, smem, st>>>(kp);
   CK(cudaGetLastError());
   h->launches++;
   return MPC_OK;
 }
 
-template <int NS, int MINB>
+template <int NS, int MINB, bool WARM>
 static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   static thread_local int cached_dev = -1;
   if (cached_dev != h->device) {
-    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
     cached_dev = h->device;
   }
   int threads = h->lane_threads;           // 0 = automatic
@@ -495,8 +504,8 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
     if (threads > MPC_LANE_SM_STRIDE) threads = MPC_LANE_SM_STRIDE;
     static thread_local int cached_dev_h = -1;
     if (cached_dev_h != h->device) {
-      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
-      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
+      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
+      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
       cached_dev_h = h->device;
     }
   }
@@ -539,11 +548,11 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   }
   if (!h->d_ckpt) {
     // no record buffers at all: one launch, hand-overs go through the restart list
-    mpc_lane_kernel<NS, MINB, false><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
+    mpc_lane_kernel<NS, MINB, false, WARM><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
     CK(cudaGetLastError());
     h->launches++;
     h->pre_recorded = false;
-    return launch_finisher<NS>(h, kp, st, kp.B);
+    return launch_finisher<NS, WARM>(h, kp, st, kp.B);
   }
   cap = h->cap_ckpt;
   double *buf[2] = {h->d_ckpt, h->d_ckpt + h->cap_ckpt * rec};
@@ -552,7 +561,7 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   kp.park_lanes = park; kp.handoff_iter = rule1 ? h->handoff_iter : INT_MAX;
   kp.chain_counts = cnt; kp.chain_buf0 = buf[0]; kp.chain_buf1 = buf[1];
   kp.chain_pos = 0; kp.chain_last = phases + 1; kp.resume_min = h->resume_min;
-  mpc_lane_kernel<NS, MINB, false><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
+  mpc_lane_kernel<NS, MINB, false, WARM><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
   CK(cudaGetLastError());
   h->launches++;
   // resume launches: enough lanes for a full buffer in one pass, dealt over all SMs.  Each works out on the device
@@ -567,7 +576,7 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   kp.ckpt = nullptr; kp.ckpt_count = nullptr;
   for (int k = 1; k <= phases; k++) {
     kp.chain_pos = k;
-    mpc_lane_kernel<NS, MINB, true><<<(unsigned)rgrid, rthreads, lane_smem, st>>>(kp);
+    mpc_lane_kernel<NS, MINB, true, WARM><<<(unsigned)rgrid, rthreads, lane_smem, st>>>(kp);
     CK(cudaGetLastError());
     h->launches++;
   }
@@ -580,11 +589,11 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
     h->pre_kp = kp;
     h->pre_rec = (int)Lane<NS, false>::CK_SIZE; h->pre_cki = (int)Lane<NS, false>::CK_I;
   }
-  return launch_finisher<NS>(h, kp, st, (long long)kp.B < (long long)cap * 2 ? kp.B : (long long)cap * 2);
+  return launch_finisher<NS, WARM>(h, kp, st, (long long)kp.B < (long long)cap * 2 ? kp.B : (long long)cap * 2);
 }
 
 // The coop kernel: one problem per group of 16 or 32 lanes, per-stage rows in shared memory.
-template <int NS>
+template <int NS, bool WARM>
 static int launch_coop(mpc_handle *h, KParams &kp, cudaStream_t st) {
   const int threads = 128;
   const int G = NS <= 16 ? 16 : 32;
@@ -592,8 +601,8 @@ static int launch_coop(mpc_handle *h, KParams &kp, cudaStream_t st) {
   const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
   static thread_local int cached_dev = -1, per_sm = 0;
   if (cached_dev != h->device) {
-    CK(cudaFuncSetAttribute(mpc_coop_kernel<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_kernel<NS>, threads, smem));
+    CK(cudaFuncSetAttribute(mpc_coop_kernel<NS, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_kernel<NS, WARM>, threads, smem));
     cached_dev = h->device;
   }
   if (per_sm < 1) { snprintf(g_err, sizeof(g_err), "coop kernel does not fit on an SM (smem %zu)", smem); return MPC_ECUDA; }
@@ -605,15 +614,77 @@ static int launch_coop(mpc_handle *h, KParams &kp, cudaStream_t st) {
   int rc = ensure_coop_scratch<NS>(h, kp, grid * groups);
   if (rc) return rc;
   if (kp.counter) CK(cudaMemsetAsync(kp.counter, 0, sizeof(int), st));
-  mpc_coop_kernel<NS><<<(unsigned)grid, threads, smem, st>>>(kp);
+  mpc_coop_kernel<NS, WARM><<<(unsigned)grid, threads, smem, st>>>(kp);
   CK(cudaGetLastError());
   h->launches++;
   return MPC_OK;
 }
 
+// warm-started launches run their own instantiations of the kernels (Lane::init)
+template <int NS>
+static int launch_coop_ws(mpc_handle *h, KParams &kp, cudaStream_t st) {
+  return kp.ws_x ? launch_coop<NS, true>(h, kp, st) : launch_coop<NS, false>(h, kp, st);
+}
+template <int NS, int MINB>
+static int launch_lane_ws(mpc_handle *h, KParams &kp, cudaStream_t st) {
+  return kp.ws_x ? launch_lane<NS, MINB, true>(h, kp, st) : launch_lane<NS, MINB, false>(h, kp, st);
+}
+
 extern "C" int mpc_set_dual_outputs(mpc_handle *h, double *lambda, double *zl, double *zu) {
   if (!h || ((lambda != nullptr) != (zl != nullptr)) || ((lambda != nullptr) != (zu != nullptr))) return MPC_EINVAL;
   h->dual_lam = lambda; h->dual_zl = zl; h->dual_zu = zu;
+  return MPC_OK;
+}
+
+extern "C" int mpc_set_warm_start(mpc_handle *h, const double *x0, const double *lambda0, const double *zl0,
+                                  const double *zu0, double mu_init) {
+  if (!h || !(mu_init >= 0.0) || mu_init == INFINITY) return MPC_EINVAL;
+  h->ws_x = x0;
+  h->ws_lam = x0 ? lambda0 : nullptr; h->ws_zl = x0 ? zl0 : nullptr; h->ws_zu = x0 ? zu0 : nullptr;
+  h->ws_mu = mu_init > 0.0 ? mu_init : 0.1;   // Ipopt's mu_init default
+  return MPC_OK;
+}
+
+// Receding-horizon shift, one thread per problem: every block of stages of the layouts of `full` and of the multiplier
+// outputs moves one stage earlier.  The new last stage of a state block continues with the increment of the old last
+// stage (the model's step with the last stage's rates held: the shift needs neither the polynomial nor dt, and uses
+// only additions, so that a CPU restatement gives the same bits); actuations and multipliers repeat their last stage.
+__global__ void mpc_warm_start_shift_kernel(int B, int N, const double *x, const double *lam, const double *zl,
+                                            const double *zu, double *x0, double *lam0, double *zl0, double *zu0) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const size_t sB = (size_t)B;
+  auto shift = [&](const double *in, double *out, int r0, int n, bool extrapolate) {
+    for (int i = 0; i + 1 < n; i++) out[(size_t)(r0 + i) * sB + b] = in[(size_t)(r0 + i + 1) * sB + b];
+    const double last = in[(size_t)(r0 + n - 1) * sB + b];
+    out[(size_t)(r0 + n - 1) * sB + b] = extrapolate ? __dadd_rn(last, __dsub_rn(last, in[(size_t)(r0 + n - 2) * sB + b])) : last;
+  };
+  // x, y, psi, v, cte, epsi: N stages from row k*N; delta, a: N-1 stages from rows 6N, 7N-1 (MPC.cpp:189-196)
+  for (int k = 0; k < 6; k++) shift(x, x0, k * N, N, true);
+  shift(x, x0, 6 * N, N - 1, false);
+  shift(x, x0, 7 * N - 1, N - 1, false);
+  if (lam)
+    for (int k = 0; k < 6; k++) shift(lam, lam0, k * N, N, false);
+  const double *zin[2] = {zl, zu};
+  double *zout[2] = {zl0, zu0};
+  for (int j = 0; j < 2; j++) {
+    if (!zin[j]) continue;
+    for (int k = 0; k < 6; k++) shift(zin[j], zout[j], k * N, N, false);
+    shift(zin[j], zout[j], 6 * N, N - 1, false);
+    shift(zin[j], zout[j], 7 * N - 1, N - 1, false);
+  }
+}
+
+extern "C" int mpc_warm_start_shift(mpc_handle *h, int B, const double *x, const double *lambda, const double *zl,
+                                    const double *zu, double *x0, double *lambda0, double *zl0, double *zu0,
+                                    void *cuda_stream) {
+  if (!h || B < 0 || !x || !x0 || (!lambda != !lambda0) || (!zl != !zl0) || (!zu != !zu0)) return MPC_EINVAL;
+  if (B == 0) return MPC_OK;
+  CK(cudaSetDevice(h->device));
+  mpc_warm_start_shift_kernel<<<(B + 255) / 256, 256, 0, (cudaStream_t)cuda_stream>>>(B, h->cfg.N, x, lambda, zl, zu,
+                                                                                      x0, lambda0, zl0, zu0);
+  CK(cudaGetLastError());
+  h->launches++;
   return MPC_OK;
 }
 
@@ -655,11 +726,17 @@ static void fill_kparams(const mpc_config &c, int B, KParams &kp) {
   memcpy(kp.steer_speeds, c.steer_speeds, sizeof(kp.steer_speeds));
 }
 
-extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const double *coeffs,
-                               const double *yaw_lo, const double *yaw_hi, const double *weights,
-                               const int *N_per, const double *dt_per, double *result, double *traj_x,
-                               double *traj_y, double *full, int *status, int *iters, void *cuda_stream) {
+// a warm start is defined for the whole horizon of every problem: not with per-problem horizons
+static int check_warm_start(const mpc_handle *h, const int *N_per) { return h->ws_x && N_per ? MPC_EINVAL : MPC_OK; }
+
+// mpc_solve_batch; `warm` = the handle's warm start applies (the solves of the C-ABI's batch entry points, not the
+// single solve and the MPC::run-level entry points, whose start point stays the reference's)
+static int solve_batch(mpc_handle *h, bool warm, int B, const double *state, const double *coeffs, const double *yaw_lo,
+                       const double *yaw_hi, const double *weights, const int *N_per, const double *dt_per,
+                       double *result, double *traj_x, double *traj_y, double *full, int *status, int *iters,
+                       void *cuda_stream) {
   if (!h || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !result) return MPC_EINVAL;
+  if (warm && check_warm_start(h, N_per)) return MPC_EINVAL;
   if (B == 0) return MPC_OK;
   CK(cudaSetDevice(h->device));
   const mpc_config &c = h->cfg;
@@ -670,6 +747,9 @@ extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const 
   kp.result = result; kp.traj_x = traj_x; kp.traj_y = traj_y; kp.full = full; kp.status = status; kp.iters = iters;
   kp.counter = h->d_counter;
   kp.dual_lam = h->dual_lam; kp.dual_zl = h->dual_zl; kp.dual_zu = h->dual_zu;
+  if (warm && h->ws_x) {
+    kp.ws_x = h->ws_x; kp.ws_lam = h->ws_lam; kp.ws_zl = h->ws_zl; kp.ws_zu = h->ws_zu; kp.ws_mu = h->ws_mu;
+  }
   // Kernel choice (crossovers measured on B200, profiles/r01_kernel_crossover.txt): below MPC_LANE_MIN_BATCH
   // problems there are fewer problems than lanes and the time is set by the longest-running problem, so the
   // coop kernel (one problem per group of 16/32 lanes) wins; above it the lane kernel (one problem per lane)
@@ -681,11 +761,11 @@ extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const 
   }
   if (kind == MPC_KERNEL_COOP) {
     if (h->one_shot) kp.counter = nullptr;   // mpc_solve_one: one group, no work queue
-    if (c.N <= 10) return launch_coop<10>(h, kp, (cudaStream_t)cuda_stream);
+    if (c.N <= 10) return launch_coop_ws<10>(h, kp, (cudaStream_t)cuda_stream);
 #ifndef MPC_DEV_N10
-    if (c.N <= 20) return launch_coop<20>(h, kp, (cudaStream_t)cuda_stream);
-    if (c.N <= 32) return launch_coop<32>(h, kp, (cudaStream_t)cuda_stream);
-    return launch_coop<MPC_NMAX>(h, kp, (cudaStream_t)cuda_stream);
+    if (c.N <= 20) return launch_coop_ws<20>(h, kp, (cudaStream_t)cuda_stream);
+    if (c.N <= 32) return launch_coop_ws<32>(h, kp, (cudaStream_t)cuda_stream);
+    return launch_coop_ws<MPC_NMAX>(h, kp, (cudaStream_t)cuda_stream);
 #else
     return MPC_EINVAL;   // development build (-DMPC_DEV_N10, a third of the compile time): N <= 10 only
 #endif
@@ -708,14 +788,22 @@ extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const 
     h->launches += 3;
     kp.perm = h->d_perm;
   }
-  if (c.N <= 10) return launch_lane<10, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
+  if (c.N <= 10) return launch_lane_ws<10, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
 #ifndef MPC_DEV_N10
-  if (c.N <= 20) return launch_lane<20, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-  if (c.N <= 32) return launch_lane<32, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-  return launch_lane<MPC_NMAX, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
+  if (c.N <= 20) return launch_lane_ws<20, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
+  if (c.N <= 32) return launch_lane_ws<32, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
+  return launch_lane_ws<MPC_NMAX, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
 #else
   return MPC_EINVAL;   // development build (-DMPC_DEV_N10, a third of the compile time): N <= 10 only
 #endif
+}
+
+extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const double *coeffs,
+                               const double *yaw_lo, const double *yaw_hi, const double *weights,
+                               const int *N_per, const double *dt_per, double *result, double *traj_x,
+                               double *traj_y, double *full, int *status, int *iters, void *cuda_stream) {
+  return solve_batch(h, true, B, state, coeffs, yaw_lo, yaw_hi, weights, N_per, dt_per, result, traj_x, traj_y, full,
+                     status, iters, cuda_stream);
 }
 
 // Early copy-back: the outputs of the problems the final launch of a chain finished, written again -- straight into
@@ -770,7 +858,7 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
                                     const double *yaw_lo, const double *yaw_hi, const double *weights,
                                     const int *N_per, const double *dt_per, double *result, double *traj_x,
                                     double *traj_y, double *full, int *status, int *iters) {
-  if (!h || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !result) return MPC_EINVAL;
+  if (!h || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !result || check_warm_start(h, N_per)) return MPC_EINVAL;
   if (B == 0) return MPC_OK;
   CK(cudaSetDevice(h->device));
   const int N = h->cfg.N;
@@ -847,7 +935,7 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
     if (full) CK(cudaMemcpyAsync(d_full, full, (8 * (size_t)N - 2) * sB, cudaMemcpyHostToDevice, st));
   }
   h->want_pre = early; h->pre_recorded = false;
-  rc = mpc_solve_batch(h, B, (const double *)u_state, (const double *)u_coef, (const double *)u_ylo, (const double *)u_yhi,
+  rc = solve_batch(h, true, B, (const double *)u_state, (const double *)u_coef, (const double *)u_ylo, (const double *)u_yhi,
                        (const double *)u_w, (const int *)u_N, (const double *)u_dt, d_res, traj_x ? d_tx : nullptr, traj_y ? d_ty : nullptr,
                        full ? d_full : nullptr, d_status, d_iters, st);
   h->want_pre = false;
@@ -908,6 +996,8 @@ extern "C" int mpc_solve_batch_multi(mpc_multi *m, int B, const double *state, c
                                      const int *N_per, const double *dt_per, double *result, double *traj_x,
                                      double *traj_y, double *full, int *status, int *iters) {
   if (!m || m->n < 1 || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !result) return MPC_EINVAL;
+  for (int g = 0; g < m->n; g++)
+    if (check_warm_start(m->h[g], N_per)) return MPC_EINVAL;
   if (B == 0) return MPC_OK;
   const int G = m->n;
   const int N = m->h[0]->cfg.N;
@@ -948,7 +1038,7 @@ extern "C" int mpc_solve_batch_multi(mpc_multi *m, int B, const double *state, c
       if (full) CK(in2d(d_full, full, 8 * N - 2));
     }
     h->want_pre = false;
-    rc = mpc_solve_batch(h, Bs, d_state, d_coef, d_ylo, d_yhi, weights ? d_w : nullptr, N_per ? d_N : nullptr,
+    rc = solve_batch(h, true, Bs, d_state, d_coef, d_ylo, d_yhi, weights ? d_w : nullptr, N_per ? d_N : nullptr,
                          dt_per ? d_dt : nullptr, d_res, traj_x ? d_tx : nullptr, traj_y ? d_ty : nullptr,
                          full ? d_full : nullptr, d_status, d_iters, st);
     if (rc) return rc;
@@ -972,6 +1062,14 @@ extern "C" int mpc_solve_batch_multi(mpc_multi *m, int B, const double *state, c
   return first_error;
 }
 
+extern "C" int mpc_set_warm_start_one(mpc_handle *h, int on, double mu_init) {
+  if (!h || !(mu_init >= 0.0) || mu_init == INFINITY) return MPC_EINVAL;
+  h->one_warm = on != 0;
+  h->one_prev_ok = false;
+  h->one_mu = mu_init;
+  return MPC_OK;
+}
+
 // One problem, host pointers.
 extern "C" int mpc_solve_one(mpc_handle *h, const double *state, const double *coeffs, double yaw_lo,
                              double yaw_hi, double *result, double *traj_x, double *traj_y, int *status,
@@ -991,12 +1089,43 @@ extern "C" int mpc_solve_one(mpc_handle *h, const double *state, const double *c
   // one synchronisation, no copy calls -- a single solve is latency-bound and every API call counts.
   double *ho = hp + 16;
   int *hi = reinterpret_cast<int *>(hp + 16 + 9 + 2 * (size_t)N);
+  double *full = nullptr;
+  bool warm = false;
+  const double *ws_save[4] = {h->ws_x, h->ws_lam, h->ws_zl, h->ws_zu};
+  double *dual_save[3] = {h->dual_lam, h->dual_zl, h->dual_zu};
+  const double ws_mu_save = h->ws_mu;
+  if (h->one_warm) {
+    // the last solution and the next start point, each [x 8N-2 | lambda 6N | zl 8N-2 | zu 8N-2] (B = 1): the solve
+    // writes the first, the shift turns it into the second
+    const size_t nx = 8 * (size_t)N - 2, per = 3 * nx + 6 * (size_t)N;
+    if (!h->d_one || h->one_N != N) {
+      cudaFree(h->d_one);
+      h->d_one = nullptr; h->one_N = 0; h->one_prev_ok = false;
+      CK(cudaMalloc(&h->d_one, 2 * per * sizeof(double)));
+      CK(cudaMemsetAsync(h->d_one, 0, 2 * per * sizeof(double), st));   // bound multipliers of unbounded variables stay 0
+      h->one_N = N;
+    }
+    double *sol = h->d_one, *nxt = h->d_one + per;
+    full = sol;
+    h->dual_lam = sol + nx; h->dual_zl = sol + nx + 6 * N; h->dual_zu = sol + 2 * nx + 6 * N;
+    if (h->one_prev_ok) {
+      rc = mpc_warm_start_shift(h, 1, sol, sol + nx, sol + nx + 6 * N, sol + 2 * nx + 6 * N, nxt, nxt + nx,
+                                nxt + nx + 6 * N, nxt + 2 * nx + 6 * N, st);
+      if (rc) { h->dual_lam = dual_save[0]; h->dual_zl = dual_save[1]; h->dual_zu = dual_save[2]; return rc; }
+      h->ws_x = nxt; h->ws_lam = nxt + nx; h->ws_zl = nxt + nx + 6 * N; h->ws_zu = nxt + 2 * nx + 6 * N;
+      h->ws_mu = h->one_mu > 0.0 ? h->one_mu : 0.1;
+      warm = true;
+    }
+  }
   h->one_shot = true;
-  rc = mpc_solve_batch(h, 1, hp, hp + 6, hp + 11, hp + 12, nullptr, nullptr, nullptr, ho, ho + 9, ho + 9 + N, nullptr, hi,
-                       hi + 1, st);
+  rc = solve_batch(h, warm, 1, hp, hp + 6, hp + 11, hp + 12, nullptr, nullptr, nullptr, ho, ho + 9, ho + 9 + N, full, hi,
+                   hi + 1, st);
   h->one_shot = false;
+  h->ws_x = ws_save[0]; h->ws_lam = ws_save[1]; h->ws_zl = ws_save[2]; h->ws_zu = ws_save[3]; h->ws_mu = ws_mu_save;
+  h->dual_lam = dual_save[0]; h->dual_zl = dual_save[1]; h->dual_zu = dual_save[2];
   if (rc) return rc;
   CK(cudaStreamSynchronize(st));
+  if (h->one_warm) h->one_prev_ok = hi[0] == MPC_STATUS_SUCCESS;   // a failed solve is no start point
   for (int k = 0; k < 9; k++) result[k] = ho[k];
   if (traj_x) for (int k = 0; k < N; k++) traj_x[k] = ho[9 + k];
   if (traj_y) for (int k = 0; k < N; k++) traj_y[k] = ho[9 + N + k];
@@ -1141,7 +1270,7 @@ extern "C" int mpc_run_batch(mpc_handle *h, int B, const double *pose, const dou
   const int thr = 128, grid = (B + thr - 1) / thr;
   mpc_run_pre_kernel<<<grid, thr, 0, st>>>(h->cfg, R);
   CK(cudaGetLastError());
-  rc = mpc_solve_batch(h, B, R.state, R.coeffs, R.yaw_lo, R.yaw_hi, nullptr, nullptr, nullptr, result, traj_x, traj_y,
+  rc = solve_batch(h, false, B, R.state, R.coeffs, R.yaw_lo, R.yaw_hi, nullptr, nullptr, nullptr, result, traj_x, traj_y,
                        nullptr, d_status, d_iters, st);
   if (rc) return rc;
   mpc_run_post_kernel<<<grid, thr, 0, st>>>(h->cfg, B, R.aux, result, out8);
@@ -1220,7 +1349,7 @@ extern "C" int mpc_rollout(mpc_handle *h, int V, int T, const double *track_x, c
   for (int k = 0; k < T; k++) {
     A.step = k;
     mpc_loop_pre_kernel<<<grid, thr, 0, st>>>(h->cfg, A);
-    rc = mpc_solve_batch(h, V, A.state, A.coeffs, A.yaw_lo, A.yaw_hi, nullptr, nullptr, nullptr, A.result, nullptr,
+    rc = solve_batch(h, false, V, A.state, A.coeffs, A.yaw_lo, A.yaw_hi, nullptr, nullptr, nullptr, A.result, nullptr,
                          nullptr, nullptr, d_status, d_iters, st);
     if (rc) return rc;
     mpc_loop_post_kernel<<<grid, thr, 0, st>>>(h->cfg, A);

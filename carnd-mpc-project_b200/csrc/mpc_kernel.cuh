@@ -102,7 +102,17 @@ struct KParams {
   // coop kernels: global scratch per lane group (watchdog backup, restoration-phase rows), scratch_stride doubles each
   double *scratch;
   long long scratch_stride;
+  // warm start (mpc_set_warm_start): start point in the layouts of `full` and of the multiplier outputs, unscaled
+  // problem; ws_x == NULL is a cold start.  ws_lam / ws_zl / ws_zu may be NULL (cold-start estimate of that part).
+  // ws_mu: the initial barrier parameter of a warm start (Ipopt's mu_init).
+  const double *ws_x, *ws_lam, *ws_zl, *ws_zu;
+  double ws_mu;
 };
+
+// Ipopt's warm_start_init_point options at their defaults (IpWarmStartIterInitializer)
+#define K_WS_BOUND_PUSH 1e-3        // warm_start_bound_push
+#define K_WS_BOUND_FRAC 1e-3        // warm_start_bound_frac
+#define K_WS_MULT_BOUND_PUSH 1e-3   // warm_start_mult_bound_push
 
 // ------------------------------------------------------------------------------------------------
 // group (G lanes) collectives: xor butterflies give every lane the bit-identical result, which

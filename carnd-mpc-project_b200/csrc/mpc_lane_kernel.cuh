@@ -180,6 +180,9 @@ struct Lane {
   // problem set-up: MPC.cpp:204-281 (start point, bounds), frozen branches of FG_eval at the
   // start point (MPC.cpp:72,79,87,89), Ipopt's objective scaling and bound relaxation / push
   // ------------------------------------------------------------------------------------------
+  // WARM: the kernel is instantiated for warm-started launches (KParams::ws_x); the cold instantiations compile to
+  // the code they had before the warm start existed (the persistent lane kernel is sensitive to its code size)
+  template <bool WARM = false>
   __device__ void init(const KParams &P, int b_) {
     b = b_;
     const int B = P.B;
@@ -265,6 +268,61 @@ struct Lane {
     force_accept = false; wd_skip = false; was_tiny = false; wd_trial = 0; trips = 0;
     tiny_tol = P.tiny_step_tol;
     mode = LM_EV0;
+    gsync();
+    if (WARM && P.ws_x) warm_init(P);
+  }
+  // Ipopt's warm_start_init_point: the caller's primal point pushed into the bounds with warm_start_bound_push /
+  // warm_start_bound_frac (the formula of the cold start with 1e-3 for 1e-2), the caller's multipliers taken over to
+  // the gradient-scaled problem -- times the objective factor sf, the factor write_outputs divides out; constraints
+  // and variables are not scaled -- with the bound multipliers raised to at least warm_start_mult_bound_push.
+  // lambda without a caller's value is the least-squares estimate (trip_accept), zl / zu without one stay at 1.
+  // The scaling factor and the frozen branches of FG_eval stay those of the problem's own start point (above), so
+  // a warm-started solve iterates on the same scaled problem as a cold one.
+  __device__ void warm_init(const KParams &P) {
+    const size_t B = (size_t)P.B;
+    const int Nf = P.Nmax;
+    const double sf = PC[LC_SF];
+    double pl[4], pu[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      const double lo = PC[LC_LO + k], hi = PC[LC_HI + k], span = hi - lo;
+      pl[k] = fmin(K_WS_BOUND_PUSH * fmax(1.0, fabs(lo)), K_WS_BOUND_FRAC * span);
+      pu[k] = fmin(K_WS_BOUND_PUSH * fmax(1.0, fabs(hi)), K_WS_BOUND_FRAC * span);
+    }
+    // rows of the reference's layout (MPC.cpp:189-196) holding psi, v, delta, a of stage i
+    const int zrow[4] = {2 * Nf, 3 * Nf, 6 * Nf, 7 * Nf - 1};
+#pragma unroll 1
+    for (int i = g0; i < N; i += gstep) {
+      const bool hasu = i < N - 1;
+      double v[8];
+#pragma unroll
+      for (int k = 0; k < 6; k++) v[k] = P.ws_x[(size_t)(k * Nf + i) * B + b];
+      v[6] = hasu ? P.ws_x[(size_t)(6 * Nf + i) * B + b] : ST[i][ST_U + 0];
+      v[7] = hasu ? P.ws_x[(size_t)(7 * Nf - 1 + i) * B + b] : ST[i][ST_U + 1];
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        double &x = v[k < 2 ? k + 2 : k + 4];
+        if (k >= 2 && !hasu) continue;
+        if (x < PC[LC_LO + k] + pl[k]) x = PC[LC_LO + k] + pl[k];
+        if (x > PC[LC_HI + k] - pu[k]) x = PC[LC_HI + k] - pu[k];
+      }
+#pragma unroll
+      for (int k = 0; k < 6; k++) ST[i][ST_S + k] = v[k];
+      ST[i][ST_U + 0] = v[6]; ST[i][ST_U + 1] = v[7];
+      if (P.ws_lam) {
+#pragma unroll
+        for (int k = 0; k < 6; k++) ST[i][ST_LAM + k] = P.ws_lam[(size_t)(k * Nf + i) * B + b] * sf;
+      }
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        if (k >= 2 && !hasu) continue;
+        const size_t at = (size_t)(zrow[k] + i) * B + b;
+        if (P.ws_zl) ST[i][ST_ZL + k] = fmax(P.ws_zl[at] * sf, K_WS_MULT_BOUND_PUSH);
+        if (P.ws_zu) ST[i][ST_ZU + k] = fmax(P.ws_zu[at] * sf, K_WS_MULT_BOUND_PUSH);
+      }
+    }
+    mu = P.ws_mu;
+    tau = fmax(K_TAU_MIN, 1.0 - mu);
     gsync();
   }
   // BacktrackingLineSearch::Reset (at every change of the barrier parameter): empty filter, no watchdog
@@ -2839,6 +2897,7 @@ struct Lane {
     return true;
   }
   // slot 2: acceptance logic, then the sweep that accepts the step and measures the KKT error
+  template <bool WARM = false>
   __device__ __forceinline__ void trip_accept(const KParams &P) {
     bool upd = false, lsq = false, zero = false, err = false;
     if (m1 == LM_EV0) {
@@ -2922,12 +2981,14 @@ struct Lane {
     if (flags) {
       advance(upd, lsq, zero);
       if (upd) { fx = ft; lsum = lt; theta = tht; }
-      if (m1 == LM_EV0) {
+      if (m1 == LM_EV0 && !(WARM && P.ws_lam)) {
         mode = LM_LSQ;
       } else if (lsq && !(lsq_lmax <= K_CONSTR_MULT_INIT_MAX)) {
         mode = LM_LSQ_ZERO;
       } else {
-        if (upd) iter++;
+        // (a warm start with the caller's lambda goes from the start point straight to the convergence test: the
+        // sweep above has measured the errors there with those multipliers)
+        if (upd && !(WARM && m1 == LM_EV0)) iter++;
         if (FULL && was_tiny) {
           // the second tiny step in a row with a small dual step asks for a smaller barrier parameter
           if (tiny_last && dy_max < K_TINY_STEP_Y_TOL) tiny_flag = true;
@@ -2946,11 +3007,12 @@ struct Lane {
   // coop kernels: trips until the problem is finished.  Every iteration costs a handful of trips (one in the common
   // case, a few with inertia correction, second-order corrections or backtracking); a problem that has taken 64 trips
   // per allowed iteration is not making progress and ends as an internal error instead of holding the device.
+  template <bool WARM = false>
   __device__ __forceinline__ void run_to_completion(const KParams &P) {
     long long budget = 64LL * (long long)(P.max_iter + 16);
     while (mode != LM_FINISH) {
       trip_eval();
-      trip_accept(P);
+      trip_accept<WARM>(P);
       if (mode == LM_FINISH) break;
       trip_factor();
       trip_solve(P);
@@ -3079,7 +3141,8 @@ template <class T> __device__ __forceinline__ void lane_rows_attach(T &, double 
 #ifndef MPC_LANE_MAXT
 #define MPC_LANE_MAXT 256   // largest CTA the lane kernel is compiled for (register cap = 65536 / (MAXT * MINB)): experiments only
 #endif
-template <int NS, int MINB, bool RESUME>
+// WARM: launches with a warm start (Lane::init); a resume launch may hold a warm problem parked before its first trip
+template <int NS, int MINB, bool RESUME, bool WARM>
 #ifdef MPC_LANE_MAXNREG
 __global__ void __maxnreg__(MPC_LANE_MAXNREG) mpc_lane_kernel(const KParams P) {
 #else
@@ -3142,7 +3205,7 @@ __global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KPa
           else Z.mode = LM_DONE;
         } else {
           const int nb = atomicAdd(P.counter, 1);
-          if (nb < P.B) Z.init(P, P.perm ? P.perm[nb] : nb); else Z.mode = LM_DONE;
+          if (nb < P.B) Z.template init<WARM>(P, P.perm ? P.perm[nb] : nb); else Z.mode = LM_DONE;
         }
       }
     }
@@ -3155,7 +3218,7 @@ __global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KPa
 #endif
     if (__syncthreads_and(Z.mode == LM_DONE)) break;
     Z.trip_eval();
-    Z.trip_accept(P);
+    Z.template trip_accept<WARM>(P);
     Z.trip_factor();
     Z.trip_solve(P);
     // progress guard (see run_to_completion): a problem that stops making progress must not hold the whole grid
@@ -3173,7 +3236,7 @@ __global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KPa
 // reads.  A trip takes a fraction of the time a lone lane needs, which is what matters when there are
 // fewer problems than lanes: single solves (MPC::solve called once per telemetry message), closed-loop
 // steps of a few thousand vehicles, and the last long-running problems of a big batch.
-template <int NS>
+template <int NS, bool WARM>
 __global__ void __launch_bounds__(128, 2) mpc_coop_kernel(const KParams P) {
   extern __shared__ double coop_smem[];
   const int G = Lane<NS, true>::NS_GROUP;
@@ -3194,8 +3257,8 @@ __global__ void __launch_bounds__(128, 2) mpc_coop_kernel(const KParams P) {
       nb = pass++ ? P.B : (int)((blockIdx.x * blockDim.x + threadIdx.x) / G);
     }
     if (nb >= P.B) break;
-    Z.init(P, nb);
-    Z.run_to_completion(P);
+    Z.template init<WARM>(P, nb);
+    Z.template run_to_completion<WARM>(P);
     if (Z.g0 == 0) Z.write_outputs(P);
     Z.gsync();
   }
@@ -3204,7 +3267,7 @@ __global__ void __launch_bounds__(128, 2) mpc_coop_kernel(const KParams P) {
 // The coop kernel on the problems the lane kernel parked or handed over: each group takes a record, restores the
 // state and carries on from the trip where the lane stopped; then the problems that were handed over when no record
 // slot was free (restart_list) are solved from the start.
-template <int NS>
+template <int NS, bool WARM>
 #ifndef MPC_COOP_RESUME_MINB
 #define MPC_COOP_RESUME_MINB 2   // CTAs per SM the finisher is compiled for at N <= 10 (3 = 168 registers: experiment)
 #endif
@@ -3238,8 +3301,8 @@ __global__ void __launch_bounds__(128, NS <= 10 ? MPC_COOP_RESUME_MINB : 2) mpc_
       k = __shfl_sync(Z.gm, k, 0, G);
       if (k >= cnt) break;
       if (phase == 0) Z.load(rec_in + (size_t)k * Lane<NS, true>::CK_SIZE);
-      else Z.init(P, P.restart_list[k]);
-      Z.run_to_completion(P);
+      else Z.template init<WARM>(P, P.restart_list[k]);
+      Z.template run_to_completion<WARM>(P);
       if (Z.g0 == 0) Z.write_outputs(P);
       Z.gsync();
     }

@@ -225,11 +225,43 @@ int mpc_tail_counts(mpc_handle *h, int *parked, int n);
  * reference's NLP independently of the solver.  All NULL switches the outputs off.  Only with N_per == NULL. */
 int mpc_set_dual_outputs(mpc_handle *h, double *lambda, double *zl, double *zu);
 
+/* Warm start (Ipopt's warm_start_init_point) for the following mpc_solve_batch / _host / _multi calls on this handle
+ * (lane and coop kernels; mpc_run_batch and mpc_rollout start cold; mpc_solve_one: mpc_set_warm_start_one).  DEVICE buffers on the
+ * handle's device, in the layouts of the outputs, for the UNSCALED problem (what `full` and mpc_set_dual_outputs
+ * return, so that a solution can be fed straight back):
+ *   x0      [8*cfg.N-2][B]  solution.x as `full` (MPC.cpp:189-196), SI units, radians
+ *   lambda0 [6*cfg.N][B]    solution.lambda as mpc_set_dual_outputs, or NULL: least-squares estimate as a cold start
+ *   zl0, zu0 [8*cfg.N-2][B] solution.zl / zu as mpc_set_dual_outputs, or NULL: 1 (bound_mult_init_val) as a cold start
+ * The point is pushed into the bounds with warm_start_bound_push = warm_start_bound_frac = 1e-3, the bound multipliers
+ * are raised to warm_start_mult_bound_push = 1e-3 (Ipopt's defaults).  mu_init replaces Ipopt's initial barrier
+ * parameter 0.1 for these solves (0 = keep 0.1; < 0 is MPC_EINVAL): a start point near the solution only helps
+ * with a small one.  x0 NULL switches the warm start off (the default); the multiplier pointers are then ignored.
+ * The buffers are bound to the handle and read by every later solve, so they must hold B columns for the B of that
+ * solve -- for mpc_solve_batch_multi, bind each shard's handle (mpc_multi_handle(m, g)) to buffers of that shard's
+ * [g*B/G, (g+1)*B/G) problems on its device.  Only with N_per == NULL: a solve with N_per and a warm start set
+ * returns MPC_EINVAL. */
+int mpc_set_warm_start(mpc_handle *h, const double *x0, const double *lambda0, const double *zl0, const double *zu0,
+                       double mu_init);
+/* Receding-horizon shift, asynchronous on cuda_stream (DEVICE pointers, layouts as above): from a solution (x,
+ * lambda, zl, zu) write the next control step's start point (x0, lambda0, zl0, zu0): stages 1..N-1 move to 0..N-2;
+ * the new last stage of the states continues with the increment of the old last stage, actuations and multipliers
+ * repeat their last stage.  lambda / zl / zu may each be NULL together with its output.  No output may alias
+ * another array of the call. */
+int mpc_warm_start_shift(mpc_handle *h, int B, const double *x, const double *lambda, const double *zl,
+                         const double *zu, double *x0, double *lambda0, double *zl0, double *zu0, void *cuda_stream);
+
 /* One problem, host pointers: state[6], coeffs[5] -> result[9], traj_x/traj_y[N] (or NULL).
  * What `MPC::solve` calls once per telemetry message. */
 int mpc_solve_one(mpc_handle *h, const double *state, const double *coeffs,
                   double yaw_lo, double yaw_hi,
                   double *result, double *traj_x, double *traj_y, int *status, int *iters);
+/* Warm start of mpc_solve_one (off by default): with on != 0 the handle keeps each mpc_solve_one solution (x and
+ * multipliers) on its device and starts the next mpc_solve_one from it, moved one stage on as mpc_warm_start_shift
+ * does, with initial barrier parameter mu_init (0 = 0.1).  The first call after switching on, a call after a solve
+ * that did not succeed and a call after mpc_set_config start cold.  The point stays in the previous call's
+ * coordinates: it suits problems that share a frame; MPC::run re-expresses every problem in the vehicle's frame, so
+ * there the primal start point is off by the vehicle's own motion. */
+int mpc_set_warm_start_one(mpc_handle *h, int on, double mu_init);
 /* Latency of mpc_solve_one measured in native code: `reps` calls after `warmup`, problem k % n of the given set
  * ([n][6] states, [n][MPC_NCOEF] coefficients, row-major), host clock around each call; median and 99th percentile
  * in microseconds.  bench.py reports it beside the latency seen through the Python binding. */

@@ -61,6 +61,14 @@ class MPC {
     cfg_ = cfg;
   }
 
+  // Opt-in warm start of solve() (off by default, so a drop-in MPC behaves as the reference): the previous solution
+  // stays on the device and each solve starts from it moved one stage on (mpc_set_warm_start_one); mu_init is the
+  // initial barrier parameter of those solves (0 = Ipopt's 0.1; a start point near the solution helps with a small one).
+  void setWarmStart(bool on, double mu_init = 0.0) {
+    const int rc = mpc_set_warm_start_one(h_, on ? 1 : 0, mu_init);
+    if (rc != MPC_OK) throw std::runtime_error(std::string("mpc_set_warm_start_one failed (") + std::to_string(rc) + ")");
+  }
+
   // MPC::solve, MPC.cpp:183-325.  Returns {x1, y1, psi1, v1, cte1, epsi1, delta0, a0, cost}; appends the N
   // predicted points (stage 0 included) to *x_trajectory / *y_trajectory.  target_velocity and dir are
   // accepted and ignored, as in the reference (MPC.cpp:43-47,87,152).
