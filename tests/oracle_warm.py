@@ -147,7 +147,8 @@ def lib():
 def solve_batch_warm(cfg, probs, x, lam=None, zl=None, zu=None, n_threads=1):
     """Warm-started oracle solves (initial barrier parameter cfg.mu_init): cfg / probs as for pyoracle.solve_batch;
     x [B][8N-2], lam [B][6N], zl / zu [B][8N-2] (each of lam / zl / zu may be None), unscaled, in the layouts of
-    pyoracle.solve's z / lam / zl / zu.  -> list of B dicts with status, iters, obj, result, z, lam, zl, zu."""
+    pyoracle.solve's z / lam / zl / zu.  -> list of B dicts with status, iters, obj, result, z, lam, zl, zu and the
+    branch counters of pyoracle.solve (n_resto, n_watchdog, n_tiny, n_filter_reset, n_filter_max)."""
     from oracle import pyoracle as po
     B = len(probs)
     n, m = 8 * cfg.N - 2, 6 * cfg.N
@@ -161,5 +162,7 @@ def solve_batch_warm(cfg, probs, x, lam=None, zl=None, zu=None, n_threads=1):
     out = (po.OrcResult * B)()
     lib().orc_solve_batch_warm(C.byref(cfg), probs, warm, B, out, n_threads)
     return [{"status": r.status, "iters": r.iters, "obj": r.obj, "result": np.array(r.result[:9]),
-             "z": np.array(r.z[:n]), "lam": np.array(r.lam[:m]), "zl": np.array(r.zl[:n]), "zu": np.array(r.zu[:n])}
+             "z": np.array(r.z[:n]), "lam": np.array(r.lam[:m]), "zl": np.array(r.zl[:n]), "zu": np.array(r.zu[:n]),
+             "n_resto": r.n_resto, "n_watchdog": r.n_watchdog, "n_tiny": r.n_tiny, "n_filter_reset": r.n_filter_reset,
+             "n_filter_max": r.n_filter_max}
             for r in out]
