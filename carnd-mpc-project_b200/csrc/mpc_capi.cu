@@ -16,6 +16,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "mpc_kernel.cuh"
@@ -42,6 +43,11 @@ static int cuda_fail(cudaError_t e, const char *what) {
 // [MPC_RESTART_COUNT] problems handed to the final launch without a record, [MPC_RESTART_CURSOR] its cursor over them
 enum { MPC_MAX_PHASES = 6, MPC_RESTART_COUNT = 17, MPC_RESTART_CURSOR = 18, MPC_HIST0 = 20, MPC_NCOUNTER = MPC_HIST0 + MPC_NMAX + 1 };
 
+// a kernel whose attributes a handle has set, and its CTAs per SM (coop family; 0 for the lane kernel).  Room for every
+// instantiation: 4 horizons x (coop, finisher, lane kernel: cold and warm; rollout).
+struct KernelAttr { const void *fn; int per_sm; };
+enum { MPC_NKERNELS = 28 };
+
 struct mpc_handle {
   mpc_config cfg;
   int device;
@@ -51,7 +57,6 @@ struct mpc_handle {
   int kernel_kind;      // MPC_KERNEL_AUTO / LANE / COOP
   int lane_threads;     // threads per CTA of the lane kernel
   int lane_ctas_per_sm; // CTAs per SM of the lane kernel (0 = occupancy maximum)
-  bool one_shot;        // set by mpc_solve_one around its launch
   int handoff_iter;     // rule 1: lane kernel parks problems still running after this many iterations (0 = never, the default)
   int park_lanes;       // tail packing: a warp with at most this many problems left parks them once the queue is empty (0 = off)
   int resume_phases;    // lane-kernel resume launches between the main launch and the final one
@@ -59,10 +64,7 @@ struct mpc_handle {
   // early copy-back (mpc_solve_batch_host): the device->host copies of a lane-kernel chain start before its final launch
   cudaStream_t stream2;
   cudaEvent_t ev_pre, ev_copy;
-  bool want_pre, pre_recorded;
   bool no_early_copy;   // test switch: always copy back after the last launch
-  KParams pre_kp;       // parameters of the chain's final launch (its record list = the outputs still to come)
-  int pre_rec, pre_cki; // record size and offset of the problem index in a record
   double *d_ckpt;       // migration records, two buffers of cap_ckpt records (each launch of a chain reads one, writes the other)
   size_t cap_ckpt;      // records per buffer
   int ckpt_ns;
@@ -93,6 +95,8 @@ struct mpc_handle {
   int *d_run_i;
   size_t cap_run;
   cudaStream_t stream;
+  KernelAttr attr[MPC_NKERNELS];   // one device and one call in flight per handle: no lock
+  int n_attr;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -447,67 +451,91 @@ static int ensure_restart(mpc_handle *h, KParams &kp) {
   return MPC_OK;
 }
 
-// The lane kernel and the launches that finish its tail, all on one stream with no host round trip:
-//   main launch            fresh problems from the work queue; parks by rule 1 (iterations) and rule 2 (sparse warp)
-//   resume launches        the parked problems, 32 to a warp; park by rule 2 into the other buffer
-//   final launch           the coop kernel (one problem per lane group, rows in shared memory, every branch of the
-//                          algorithm): the records that are left, then the problems handed over without a record
-#ifndef MPC_LANE_MINB
-#define MPC_LANE_MINB 1   // CTAs per SM the lane kernel is compiled for (__launch_bounds__(256, MINB)): experiments only
+// Calls f(std::integral_constant<int, NS>()) with the horizon capacity NS of the kernels that solve horizon N.
+template <class F>
+static int with_horizon(int N, F f) {
+  if (N <= 10) return f(std::integral_constant<int, 10>());
+#ifndef MPC_DEV_N10
+  if (N <= 20) return f(std::integral_constant<int, 20>());
+  if (N <= 32) return f(std::integral_constant<int, 32>());
+  return f(std::integral_constant<int, MPC_NMAX>());
+#else
+  return MPC_EINVAL;   // development build (-DMPC_DEV_N10, a third of the compile time): N <= 10 only
 #endif
-// the final launch of a lane-kernel chain: the coop kernel on the parked / handed-over records and the restart list
-template <int NS, bool WARM>
-static int launch_finisher(mpc_handle *h, KParams &kp, cudaStream_t st, long long max_work) {
-  const int ct = 128, G = NS <= 16 ? 16 : 32, groups = ct / G;
-  const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
-  static thread_local int cached_dev2 = -1;
-  if (cached_dev2 != h->device) {
-    CK(cudaFuncSetAttribute(mpc_coop_resume_kernel<NS, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cached_dev2 = h->device;
-  }
-  int per_sm = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_resume_kernel<NS, WARM>, ct, smem));
-  if (per_sm < 1) per_sm = 1;
-  long long g2 = (long long)h->sm_count * per_sm, w2 = (max_work + groups - 1) / groups;
-  if (g2 > w2) g2 = w2;
-  if (g2 < 1) g2 = 1;
-  int rc = ensure_coop_scratch<NS>(h, kp, g2 * groups);
+}
+
+// Sets the attributes of kernel `fn` through set(&per_sm) the first time this handle launches it; *per_sm: its CTAs
+// per SM, as `set` stored it.
+template <class Set>
+static int kernel_attrs(mpc_handle *h, const void *fn, int *per_sm, Set set) {
+  for (int i = 0; i < h->n_attr; i++)
+    if (h->attr[i].fn == fn) { *per_sm = h->attr[i].per_sm; return MPC_OK; }
+  const int rc = set(per_sm);
   if (rc) return rc;
-  mpc_coop_resume_kernel<NS, WARM><<<(unsigned)g2, ct, smem, st>>>(kp);
+  if (h->n_attr < MPC_NKERNELS) h->attr[h->n_attr++] = {fn, *per_sm};
+  return MPC_OK;
+}
+
+// The coop-family kernels (mpc_coop_kernel, mpc_coop_resume_kernel, mpc_rollout_kernel): one problem per group of 16
+// or 32 lanes, per-stage rows in shared memory, CTAs of 128 threads -- as many as fit on the SMs, but no more groups
+// than `work` problems -- and a block of global scratch per group.
+template <int NS, class Kernel, class... Args>
+static int launch_coop_family(mpc_handle *h, Kernel kernel, const char *name, KParams &kp, long long work,
+                              cudaStream_t st, const Args &...args) {
+  const int threads = 128, groups = threads / (NS <= 16 ? 16 : 32);
+  const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
+  int per_sm = 0;
+  int rc = kernel_attrs(h, (const void *)kernel, &per_sm, [&](int *n) {
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(n, kernel, threads, smem));
+    return MPC_OK;
+  });
+  if (rc) return rc;
+  if (per_sm < 1) { snprintf(g_err, sizeof(g_err), "%s does not fit on an SM (smem %zu)", name, smem); return MPC_ECUDA; }
+  long long want = (work + groups - 1) / groups, grid = (long long)h->sm_count * per_sm;
+  if (grid > want) grid = want;
+  if (grid < 1) grid = 1;
+  rc = ensure_coop_scratch<NS>(h, kp, grid * groups);
+  if (rc) return rc;
+  kernel<<<(unsigned)grid, threads, smem, st>>>(kp, args...);
   CK(cudaGetLastError());
   h->launches++;
   return MPC_OK;
 }
 
-template <int NS, int MINB, bool WARM>
-static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
-  static thread_local int cached_dev = -1;
-  if (cached_dev != h->device) {
-    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-    cached_dev = h->device;
-  }
+// What the early copy-back of mpc_solve_batch_host needs from a lane-kernel chain: whether h->ev_pre was recorded
+// before the chain's final launch, and that launch's parameters (its record list = the outputs still to come), record
+// size and offset of the problem index in a record.
+struct PreFinisher {
+  bool recorded;
+  KParams kp;
+  int rec, cki;
+};
+
+// The lane kernel and the launches that finish its tail, all on one stream with no host round trip:
+//   main launch            fresh problems from the work queue; parks by rule 1 (iterations) and rule 2 (sparse warp)
+//   resume launches        the parked problems, 32 to a warp; park by rule 2 into the other buffer
+//   final launch           the coop kernel (one problem per lane group, rows in shared memory, every branch of the
+//                          algorithm): the records that are left, then the problems handed over without a record
+// pre: NULL, or where to report the event recorded before the final launch.
+template <int NS, bool WARM>
+static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st, PreFinisher *pre) {
+  int unused;
+  int rc = kernel_attrs(h, (const void *)mpc_lane_kernel<NS, false, WARM>, &unused, [&](int *per_sm) {
+    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, false, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+    CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, true, WARM>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+    *per_sm = 0;
+    return MPC_OK;
+  });
+  if (rc) return rc;
   int threads = h->lane_threads;           // 0 = automatic
   if (threads <= 0) {
-    const long long max_lanes = (long long)h->sm_count * 256;
+    const long long max_lanes = (long long)h->sm_count * LANE_MAX_THREADS;
     const long long rounds = (kp.B + max_lanes - 1) / max_lanes;
     const long long lanes_per_sm = (kp.B + rounds * h->sm_count - 1) / (rounds * h->sm_count);
     threads = (int)((lanes_per_sm + 31) / 32) * 32;
     if (threads < 32) threads = 32;
-    if (threads > 256) threads = 256;
-  }
-  if (threads > MPC_LANE_MAXT) threads = MPC_LANE_MAXT;
-  // hybrid rows (experiment): some columns of the rows in shared memory, laid out for CTAs of at most MPC_LANE_SM_STRIDE threads
-  const bool hybrid = MPC_LANE_HYBRID(NS);
-  const size_t lane_smem = hybrid ? (size_t)NS * MPC_LANE_SM_NC * MPC_LANE_SM_STRIDE * sizeof(double) : 0;
-  if (hybrid) {
-    if (threads > MPC_LANE_SM_STRIDE) threads = MPC_LANE_SM_STRIDE;
-    static thread_local int cached_dev_h = -1;
-    if (cached_dev_h != h->device) {
-      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, false, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
-      CK(cudaFuncSetAttribute(mpc_lane_kernel<NS, MINB, true, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lane_smem));
-      cached_dev_h = h->device;
-    }
+    if (threads > LANE_MAX_THREADS) threads = LANE_MAX_THREADS;
   }
   long long want = ((long long)kp.B + threads - 1) / threads;
   long long grid = (long long)h->sm_count * (h->lane_ctas_per_sm > 0 ? h->lane_ctas_per_sm : 1);
@@ -520,10 +548,9 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   const int park = kp.B >= MPC_TAIL_MIN_BATCH ? h->park_lanes : 0;
   const int phases = park > 0 ? h->resume_phases : 0;
   int *cnt = h->d_counter + 1;   // [2k] records written by launch k of the chain, [2k + 1] cursor of the coop kernel
-  kp.ckpt = nullptr; kp.ckpt_in = nullptr; kp.ckpt_cap = 0; kp.park_lanes = 0; kp.handoff_iter = INT_MAX;
+  kp.handoff_iter = INT_MAX;
   kp.ckpt_count = cnt; kp.ckpt_next = cnt + 1; kp.ckpt_in_count = cnt;
-  kp.chain_counts = nullptr;
-  int rc = ensure_restart(h, kp);
+  rc = ensure_restart(h, kp);
   if (rc) return rc;
   CK(cudaMemsetAsync(kp.counter, 0, MPC_HIST0 * sizeof(int), st));
   // The lane kernel hands every problem that needs a rare branch of the algorithm (restoration phase, watchdog, a
@@ -548,11 +575,10 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   }
   if (!h->d_ckpt) {
     // no record buffers at all: one launch, hand-overs go through the restart list
-    mpc_lane_kernel<NS, MINB, false, WARM><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
+    mpc_lane_kernel<NS, false, WARM><<<(unsigned)grid, threads, 0, st>>>(kp);
     CK(cudaGetLastError());
     h->launches++;
-    h->pre_recorded = false;
-    return launch_finisher<NS, WARM>(h, kp, st, kp.B);
+    return launch_coop_family<NS>(h, mpc_coop_resume_kernel<NS, WARM>, "finisher", kp, kp.B, st);
   }
   cap = h->cap_ckpt;
   double *buf[2] = {h->d_ckpt, h->d_ckpt + h->cap_ckpt * rec};
@@ -561,73 +587,43 @@ static int launch_lane(mpc_handle *h, KParams &kp, cudaStream_t st) {
   kp.park_lanes = park; kp.handoff_iter = rule1 ? h->handoff_iter : INT_MAX;
   kp.chain_counts = cnt; kp.chain_buf0 = buf[0]; kp.chain_buf1 = buf[1];
   kp.chain_pos = 0; kp.chain_last = phases + 1; kp.resume_min = h->resume_min;
-  mpc_lane_kernel<NS, MINB, false, WARM><<<(unsigned)grid, threads, lane_smem, st>>>(kp);
+  mpc_lane_kernel<NS, false, WARM><<<(unsigned)grid, threads, 0, st>>>(kp);
   CK(cudaGetLastError());
   h->launches++;
   // resume launches: enough lanes for a full buffer in one pass, dealt over all SMs.  Each works out on the device
   // which buffer holds the live records (chain_resolve) and returns at once if there are too few to be worth a pass.
   int rthreads = (int)(((cap + h->sm_count - 1) / h->sm_count + 31) / 32) * 32;
-  if (rthreads > MPC_LANE_MAXT) rthreads = MPC_LANE_MAXT;
-  if (hybrid && rthreads > MPC_LANE_SM_STRIDE) rthreads = MPC_LANE_SM_STRIDE;
+  if (rthreads > LANE_MAX_THREADS) rthreads = LANE_MAX_THREADS;
   long long rgrid = ((long long)cap + rthreads - 1) / rthreads;
-  if (rgrid > (long long)h->sm_count * MPC_LANE_MINB) rgrid = (long long)h->sm_count * MPC_LANE_MINB;
+  if (rgrid > h->sm_count) rgrid = h->sm_count;
   kp.handoff_iter = INT_MAX;
   kp.perm = nullptr;
   kp.ckpt = nullptr; kp.ckpt_count = nullptr;
   for (int k = 1; k <= phases; k++) {
     kp.chain_pos = k;
-    mpc_lane_kernel<NS, MINB, true, WARM><<<(unsigned)rgrid, rthreads, lane_smem, st>>>(kp);
+    mpc_lane_kernel<NS, true, WARM><<<(unsigned)rgrid, rthreads, 0, st>>>(kp);
     CK(cudaGetLastError());
     h->launches++;
   }
   kp.chain_pos = phases + 1;
   kp.park_lanes = 0;
-  if (h->want_pre && st == h->stream) {
+  if (pre) {
     // from here on only the final launch writes outputs, and only those of the problems in its record list
     CK(cudaEventRecord(h->ev_pre, st));
-    h->pre_recorded = true;
-    h->pre_kp = kp;
-    h->pre_rec = (int)Lane<NS, false>::CK_SIZE; h->pre_cki = (int)Lane<NS, false>::CK_I;
+    pre->recorded = true;
+    pre->kp = kp;
+    pre->rec = (int)Lane<NS, false>::CK_SIZE; pre->cki = (int)Lane<NS, false>::CK_I;
   }
-  return launch_finisher<NS, WARM>(h, kp, st, (long long)kp.B < (long long)cap * 2 ? kp.B : (long long)cap * 2);
+  return launch_coop_family<NS>(h, mpc_coop_resume_kernel<NS, WARM>, "finisher", kp,
+                                (long long)kp.B < (long long)cap * 2 ? kp.B : (long long)cap * 2, st);
 }
 
 // The coop kernel: one problem per group of 16 or 32 lanes, per-stage rows in shared memory.
 template <int NS, bool WARM>
 static int launch_coop(mpc_handle *h, KParams &kp, cudaStream_t st) {
-  const int threads = 128;
-  const int G = NS <= 16 ? 16 : 32;
-  const int groups = threads / G;
-  const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
-  static thread_local int cached_dev = -1, per_sm = 0;
-  if (cached_dev != h->device) {
-    CK(cudaFuncSetAttribute(mpc_coop_kernel<NS, WARM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_coop_kernel<NS, WARM>, threads, smem));
-    cached_dev = h->device;
-  }
-  if (per_sm < 1) { snprintf(g_err, sizeof(g_err), "coop kernel does not fit on an SM (smem %zu)", smem); return MPC_ECUDA; }
-  long long want = ((long long)kp.B + groups - 1) / groups;
-  long long grid = (long long)h->sm_count * per_sm;
-  if (grid > want) grid = want;
-  if (grid < 1) grid = 1;
-  kp.ckpt = nullptr; kp.ckpt_cap = 0; kp.handoff_iter = INT_MAX; kp.ckpt_count = h->d_counter + 1; kp.ckpt_next = h->d_counter + 2;
-  int rc = ensure_coop_scratch<NS>(h, kp, grid * groups);
-  if (rc) return rc;
+  kp.handoff_iter = INT_MAX; kp.ckpt_count = h->d_counter + 1; kp.ckpt_next = h->d_counter + 2;
   if (kp.counter) CK(cudaMemsetAsync(kp.counter, 0, sizeof(int), st));
-  mpc_coop_kernel<NS, WARM><<<(unsigned)grid, threads, smem, st>>>(kp);
-  CK(cudaGetLastError());
-  h->launches++;
-  return MPC_OK;
-}
-
-// warm-started launches run their own instantiations of the kernels (Lane::init)
-template <int NS>
-static int launch_coop_ws(mpc_handle *h, KParams &kp, cudaStream_t st) {
-  return kp.ws_x ? launch_coop<NS, true>(h, kp, st) : launch_coop<NS, false>(h, kp, st);
-}
-template <int NS, int MINB>
-static int launch_lane_ws(mpc_handle *h, KParams &kp, cudaStream_t st) {
-  return kp.ws_x ? launch_lane<NS, MINB, true>(h, kp, st) : launch_lane<NS, MINB, false>(h, kp, st);
+  return launch_coop_family<NS>(h, mpc_coop_kernel<NS, WARM>, "coop kernel", kp, kp.B, st);
 }
 
 extern "C" int mpc_set_dual_outputs(mpc_handle *h, double *lambda, double *zl, double *zu) {
@@ -706,7 +702,7 @@ extern "C" int mpc_set_tail(mpc_handle *h, int park_lanes, int resume_launches, 
 
 extern "C" int mpc_set_kernel(mpc_handle *h, int kind, int lane_threads, int lane_ctas_per_sm) {
   if (!h || (kind != MPC_KERNEL_AUTO && kind != MPC_KERNEL_LANE && kind != MPC_KERNEL_COOP)) return MPC_EINVAL;
-  if (lane_threads != 0 && (lane_threads < 32 || lane_threads > 256 || lane_threads % 32)) return MPC_EINVAL;
+  if (lane_threads != 0 && (lane_threads < 32 || lane_threads > LANE_MAX_THREADS || lane_threads % 32)) return MPC_EINVAL;
   h->kernel_kind = kind;
   h->lane_threads = lane_threads;
   h->lane_ctas_per_sm = lane_ctas_per_sm < 0 ? 0 : lane_ctas_per_sm;
@@ -729,27 +725,44 @@ static void fill_kparams(const mpc_config &c, int B, KParams &kp) {
 // a warm start is defined for the whole horizon of every problem: not with per-problem horizons
 static int check_warm_start(const mpc_handle *h, const int *N_per) { return h->ws_x && N_per ? MPC_EINVAL : MPC_OK; }
 
-// mpc_solve_batch; `warm` = the handle's warm start applies (the solves of the C-ABI's batch entry points, not the
-// single solve and the MPC::run-level entry points, whose start point stays the reference's)
-static int solve_batch(mpc_handle *h, bool warm, int B, const double *state, const double *coeffs, const double *yaw_lo,
-                       const double *yaw_hi, const double *weights, const int *N_per, const double *dt_per,
-                       double *result, double *traj_x, double *traj_y, double *full, int *status, int *iters,
-                       void *cuda_stream) {
+// What one solve_batch call needs beyond the problem arrays.
+struct SolveCall {
+  const double *ws_x, *ws_lam, *ws_zl, *ws_zu;   // warm start (ws_x NULL: cold start)
+  double ws_mu;
+  double *dual_lam, *dual_zl, *dual_zu;           // multiplier outputs, or NULL
+  bool one_shot;                                  // one problem per lane group, no work queue (single solves)
+  PreFinisher *pre;                               // early copy-back: record h->ev_pre before a chain's final launch, or NULL
+};
+
+// A call with the handle's bound settings: its multiplier outputs, and its warm start if `warm` (the C-ABI's batch
+// entry points; the single solve and the MPC::run-level entry points start where the reference does).
+static SolveCall bound_call(const mpc_handle *h, bool warm) {
+  SolveCall call = {};
+  call.dual_lam = h->dual_lam; call.dual_zl = h->dual_zl; call.dual_zu = h->dual_zu;
+  if (warm && h->ws_x) {
+    call.ws_x = h->ws_x; call.ws_lam = h->ws_lam; call.ws_zl = h->ws_zl; call.ws_zu = h->ws_zu; call.ws_mu = h->ws_mu;
+  }
+  return call;
+}
+
+static int solve_batch(mpc_handle *h, const SolveCall &call, int B, const double *state, const double *coeffs,
+                       const double *yaw_lo, const double *yaw_hi, const double *weights, const int *N_per,
+                       const double *dt_per, double *result, double *traj_x, double *traj_y, double *full, int *status,
+                       int *iters, void *cuda_stream) {
   if (!h || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !result) return MPC_EINVAL;
-  if (warm && check_warm_start(h, N_per)) return MPC_EINVAL;
+  if (call.ws_x && N_per) return MPC_EINVAL;
   if (B == 0) return MPC_OK;
   CK(cudaSetDevice(h->device));
   const mpc_config &c = h->cfg;
+  cudaStream_t st = (cudaStream_t)cuda_stream;
   KParams kp;
   fill_kparams(c, B, kp);
   kp.state = state; kp.coeffs = coeffs; kp.yaw_lo = yaw_lo; kp.yaw_hi = yaw_hi; kp.weights_pp = weights;
   kp.N_pp = N_per; kp.dt_pp = dt_per;
   kp.result = result; kp.traj_x = traj_x; kp.traj_y = traj_y; kp.full = full; kp.status = status; kp.iters = iters;
   kp.counter = h->d_counter;
-  kp.dual_lam = h->dual_lam; kp.dual_zl = h->dual_zl; kp.dual_zu = h->dual_zu;
-  if (warm && h->ws_x) {
-    kp.ws_x = h->ws_x; kp.ws_lam = h->ws_lam; kp.ws_zl = h->ws_zl; kp.ws_zu = h->ws_zu; kp.ws_mu = h->ws_mu;
-  }
+  kp.dual_lam = call.dual_lam; kp.dual_zl = call.dual_zl; kp.dual_zu = call.dual_zu;
+  kp.ws_x = call.ws_x; kp.ws_lam = call.ws_lam; kp.ws_zl = call.ws_zl; kp.ws_zu = call.ws_zu; kp.ws_mu = call.ws_mu;
   // Kernel choice (crossovers measured on B200, profiles/r01_kernel_crossover.txt): below MPC_LANE_MIN_BATCH
   // problems there are fewer problems than lanes and the time is set by the longest-running problem, so the
   // coop kernel (one problem per group of 16/32 lanes) wins; above it the lane kernel (one problem per lane)
@@ -759,19 +772,9 @@ static int solve_batch(mpc_handle *h, bool warm, int B, const double *state, con
     if (c.N > 32) kind = B <= MPC_COOP_MAX_BATCH_LONG ? MPC_KERNEL_COOP : MPC_KERNEL_LANE;
     else kind = B >= MPC_LANE_MIN_BATCH ? MPC_KERNEL_LANE : MPC_KERNEL_COOP;
   }
-  if (kind == MPC_KERNEL_COOP) {
-    if (h->one_shot) kp.counter = nullptr;   // mpc_solve_one: one group, no work queue
-    if (c.N <= 10) return launch_coop_ws<10>(h, kp, (cudaStream_t)cuda_stream);
-#ifndef MPC_DEV_N10
-    if (c.N <= 20) return launch_coop_ws<20>(h, kp, (cudaStream_t)cuda_stream);
-    if (c.N <= 32) return launch_coop_ws<32>(h, kp, (cudaStream_t)cuda_stream);
-    return launch_coop_ws<MPC_NMAX>(h, kp, (cudaStream_t)cuda_stream);
-#else
-    return MPC_EINVAL;   // development build (-DMPC_DEV_N10, a third of the compile time): N <= 10 only
-#endif
-  }
-  if (N_per && B >= MPC_TAIL_MIN_BATCH && h->sort_ragged) {
-    cudaStream_t st = (cudaStream_t)cuda_stream;
+  const bool coop = kind == MPC_KERNEL_COOP;
+  if (coop && call.one_shot) kp.counter = nullptr;
+  if (!coop && N_per && B >= MPC_TAIL_MIN_BATCH && h->sort_ragged) {
     if (!h->d_perm || h->cap_perm < (size_t)B) {
       cudaFree(h->d_perm);
       h->d_perm = nullptr;
@@ -788,22 +791,24 @@ static int solve_batch(mpc_handle *h, bool warm, int B, const double *state, con
     h->launches += 3;
     kp.perm = h->d_perm;
   }
-  if (c.N <= 10) return launch_lane_ws<10, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-#ifndef MPC_DEV_N10
-  if (c.N <= 20) return launch_lane_ws<20, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-  if (c.N <= 32) return launch_lane_ws<32, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-  return launch_lane_ws<MPC_NMAX, MPC_LANE_MINB>(h, kp, (cudaStream_t)cuda_stream);
-#else
-  return MPC_EINVAL;   // development build (-DMPC_DEV_N10, a third of the compile time): N <= 10 only
-#endif
+  // warm-started launches run their own instantiations of the kernels (Lane::init)
+  auto launch = [&](auto ns, auto warm) {
+    constexpr int NS = decltype(ns)::value;
+    constexpr bool WARM = decltype(warm)::value;
+    return coop ? launch_coop<NS, WARM>(h, kp, st) : launch_lane<NS, WARM>(h, kp, st, call.pre);
+  };
+  return with_horizon(c.N, [&](auto ns) {
+    return kp.ws_x ? launch(ns, std::true_type()) : launch(ns, std::false_type());
+  });
 }
 
 extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const double *coeffs,
                                const double *yaw_lo, const double *yaw_hi, const double *weights,
                                const int *N_per, const double *dt_per, double *result, double *traj_x,
                                double *traj_y, double *full, int *status, int *iters, void *cuda_stream) {
-  return solve_batch(h, true, B, state, coeffs, yaw_lo, yaw_hi, weights, N_per, dt_per, result, traj_x, traj_y, full,
-                     status, iters, cuda_stream);
+  if (!h) return MPC_EINVAL;
+  return solve_batch(h, bound_call(h, true), B, state, coeffs, yaw_lo, yaw_hi, weights, N_per, dt_per, result, traj_x,
+                     traj_y, full, status, iters, cuda_stream);
 }
 
 // Early copy-back: the outputs of the problems the final launch of a chain finished, written again -- straight into
@@ -838,19 +843,33 @@ __global__ void mpc_patch_outputs_kernel(const KParams P, int rec_size, int cki,
 }
 
 // ---- host-pointer entry points -------------------------------------------------------------------
-static int ensure_staging(mpc_handle *h, size_t B, int N, bool with_w) {
-  if (h->d_in && h->cap_B >= B && h->cap_N >= N && (h->cap_w || !with_w)) return MPC_OK;
-  cudaFree(h->d_in); cudaFree(h->d_out); cudaFree(h->d_iout); cudaFreeHost(h->h_pin);
-  h->d_in = h->d_out = nullptr; h->d_iout = nullptr; h->h_pin = nullptr;
-  h->cap_B = 0; h->cap_N = 0; h->cap_w = false;   // a failed allocation below must not leave a capacity behind
-  size_t cap = B < 256 ? 256 : B;
-  size_t nin = (6 + 5 + 2 + 12 + 1) * cap;            // state, coeffs, yaw, weights, dt
-  size_t nout = (9 + 2 * (size_t)N + (8 * (size_t)N - 2)) * cap;
-  CK(cudaMalloc(&h->d_in, nin * sizeof(double)));
-  CK(cudaMalloc(&h->d_out, nout * sizeof(double)));
-  CK(cudaMalloc(&h->d_iout, 3 * cap * sizeof(int)));
-  CK(cudaMallocHost(&h->h_pin, 64 * sizeof(double) + (9 + 2 * (size_t)MPC_NMAX) * sizeof(double)));
-  h->cap_B = cap; h->cap_N = N; h->cap_w = true;
+// the device staging arrays of a batch of horizon N, each at stride cap_B
+struct Staging {
+  double *state, *coef, *ylo, *yhi, *w, *dt;   // inputs
+  double *res, *tx, *ty, *full;                // outputs
+  int *status, *iters, *N;
+};
+static int ensure_staging(mpc_handle *h, size_t B, int N, bool with_w, Staging *s) {
+  if (!h->d_in || h->cap_B < B || h->cap_N < N || (!h->cap_w && with_w)) {
+    cudaFree(h->d_in); cudaFree(h->d_out); cudaFree(h->d_iout); cudaFreeHost(h->h_pin);
+    h->d_in = h->d_out = nullptr; h->d_iout = nullptr; h->h_pin = nullptr;
+    h->cap_B = 0; h->cap_N = 0; h->cap_w = false;   // a failed allocation below must not leave a capacity behind
+    size_t cap = B < 256 ? 256 : B;
+    size_t nin = (6 + 5 + 2 + 12 + 1) * cap;            // state, coeffs, yaw, weights, dt
+    size_t nout = (9 + 2 * (size_t)N + (8 * (size_t)N - 2)) * cap;
+    CK(cudaMalloc(&h->d_in, nin * sizeof(double)));
+    CK(cudaMalloc(&h->d_out, nout * sizeof(double)));
+    CK(cudaMalloc(&h->d_iout, 3 * cap * sizeof(int)));
+    CK(cudaMallocHost(&h->h_pin, 64 * sizeof(double) + (9 + 2 * (size_t)MPC_NMAX) * sizeof(double)));
+    h->cap_B = cap; h->cap_N = N; h->cap_w = true;
+  }
+  if (s) {
+    const size_t cap = h->cap_B;
+    s->state = h->d_in; s->coef = s->state + 6 * cap; s->ylo = s->coef + 5 * cap; s->yhi = s->ylo + cap;
+    s->w = s->yhi + cap; s->dt = s->w + 12 * cap;
+    s->res = h->d_out; s->tx = s->res + 9 * cap; s->ty = s->tx + (size_t)N * cap; s->full = s->ty + (size_t)N * cap;
+    s->status = h->d_iout; s->iters = s->status + cap; s->N = s->iters + cap;
+  }
   return MPC_OK;
 }
 
@@ -862,14 +881,11 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
   if (B == 0) return MPC_OK;
   CK(cudaSetDevice(h->device));
   const int N = h->cfg.N;
-  int rc = ensure_staging(h, (size_t)B, N, weights != nullptr);
+  Staging d;
+  int rc = ensure_staging(h, (size_t)B, N, weights != nullptr, &d);
   if (rc) return rc;
   cudaStream_t st = h->stream;
-  const size_t cap = h->cap_B, sB = (size_t)B * sizeof(double);
-  double *d_state = h->d_in, *d_coef = d_state + 6 * cap, *d_ylo = d_coef + 5 * cap, *d_yhi = d_ylo + cap;
-  double *d_w = d_yhi + cap, *d_dt = d_w + 12 * cap;
-  double *d_res = h->d_out, *d_tx = d_res + 9 * cap, *d_ty = d_tx + (size_t)N * cap, *d_full = d_ty + (size_t)N * cap;
-  int *d_status = h->d_iout, *d_iters = d_status + cap, *d_N = d_iters + cap;
+  const size_t sB = (size_t)B * sizeof(double);
   // inputs are [k][B] with stride B on the host and on the device.  An input that lies in pinned (page-locked,
   // device-mapped) host memory is not copied: the kernels read each value once, at the start of its problem, straight
   // over PCIe -- measured free (4.61 against 4.60 ms for the 64K batch) where the copies cost 0.15 ms.  Outputs are
@@ -885,13 +901,13 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
     return cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, st);
   };
   const void *u_state, *u_coef, *u_ylo, *u_yhi, *u_w = nullptr, *u_dt = nullptr, *u_N = nullptr;
-  CK(stage(state, d_state, 6 * sB, &u_state));
-  CK(stage(coeffs, d_coef, 5 * sB, &u_coef));
-  CK(stage(yaw_lo, d_ylo, sB, &u_ylo));
-  CK(stage(yaw_hi, d_yhi, sB, &u_yhi));
-  if (weights) CK(stage(weights, d_w, 12 * sB, &u_w));
-  if (dt_per) CK(stage(dt_per, d_dt, sB, &u_dt));
-  if (N_per) CK(stage(N_per, d_N, (size_t)B * sizeof(int), &u_N));
+  CK(stage(state, d.state, 6 * sB, &u_state));
+  CK(stage(coeffs, d.coef, 5 * sB, &u_coef));
+  CK(stage(yaw_lo, d.ylo, sB, &u_ylo));
+  CK(stage(yaw_hi, d.yhi, sB, &u_yhi));
+  if (weights) CK(stage(weights, d.w, 12 * sB, &u_w));
+  if (dt_per) CK(stage(dt_per, d.dt, sB, &u_dt));
+  if (N_per) CK(stage(N_per, d.N, (size_t)B * sizeof(int), &u_N));
   // Early copy-back.  In a lane-kernel chain the final launch (the finisher) works for a quarter of the step on a few
   // thousand long-running problems; every other result is final before it starts.  If all output arrays are pinned
   // and device-mapped, the device->host copies run on a second stream beside the finisher, and a small kernel then
@@ -907,7 +923,7 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
   bool early = !h->no_early_copy;
   {
     double *hostp[4] = {result, traj_x, traj_y, full};
-    const double *devp[4] = {d_res, d_tx, d_ty, d_full};
+    const double *devp[4] = {d.res, d.tx, d.ty, d.full};
     const int rows[4] = {9, N, N, 8 * N - 2};
     for (int a = 0; a < 4 && early; a++) {
       if (!hostp[a]) continue;
@@ -915,7 +931,7 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
       if (!pa.dst[a]) early = false;
     }
     int *hosti[2] = {status, iters};
-    const int *devi[2] = {d_status, d_iters};
+    const int *devi[2] = {d.status, d.iters};
     for (int a = 0; a < 2 && early; a++) {
       if (!hosti[a]) continue;
       pa.idst[a] = (int *)mapped(hosti[a]); pa.isrc[a] = devi[a];
@@ -930,29 +946,29 @@ extern "C" int mpc_solve_batch_host(mpc_handle *h, int B, const double *state, c
   if (N_per) {
     // ragged batch: rows at or beyond a problem's horizon are left untouched by the kernels, and the copies back
     // are whole arrays -- so the staging buffers start as copies of the caller's arrays
-    if (traj_x) CK(cudaMemcpyAsync(d_tx, traj_x, (size_t)N * sB, cudaMemcpyHostToDevice, st));
-    if (traj_y) CK(cudaMemcpyAsync(d_ty, traj_y, (size_t)N * sB, cudaMemcpyHostToDevice, st));
-    if (full) CK(cudaMemcpyAsync(d_full, full, (8 * (size_t)N - 2) * sB, cudaMemcpyHostToDevice, st));
+    if (traj_x) CK(cudaMemcpyAsync(d.tx, traj_x, (size_t)N * sB, cudaMemcpyHostToDevice, st));
+    if (traj_y) CK(cudaMemcpyAsync(d.ty, traj_y, (size_t)N * sB, cudaMemcpyHostToDevice, st));
+    if (full) CK(cudaMemcpyAsync(d.full, full, (8 * (size_t)N - 2) * sB, cudaMemcpyHostToDevice, st));
   }
-  h->want_pre = early; h->pre_recorded = false;
-  rc = solve_batch(h, true, B, (const double *)u_state, (const double *)u_coef, (const double *)u_ylo, (const double *)u_yhi,
-                       (const double *)u_w, (const int *)u_N, (const double *)u_dt, d_res, traj_x ? d_tx : nullptr, traj_y ? d_ty : nullptr,
-                       full ? d_full : nullptr, d_status, d_iters, st);
-  h->want_pre = false;
+  PreFinisher pre = {};
+  SolveCall call = bound_call(h, true);
+  if (early) call.pre = &pre;
+  rc = solve_batch(h, call, B, (const double *)u_state, (const double *)u_coef, (const double *)u_ylo, (const double *)u_yhi,
+                   (const double *)u_w, (const int *)u_N, (const double *)u_dt, d.res, traj_x ? d.tx : nullptr,
+                   traj_y ? d.ty : nullptr, full ? d.full : nullptr, d.status, d.iters, st);
   if (rc) return rc;
-  const bool pre = h->pre_recorded;
-  cudaStream_t cs = pre ? h->stream2 : st;
-  if (pre) CK(cudaStreamWaitEvent(cs, h->ev_pre, 0));
-  CK(cudaMemcpyAsync(result, d_res, 9 * sB, cudaMemcpyDeviceToHost, cs));
-  if (traj_x) CK(cudaMemcpyAsync(traj_x, d_tx, (size_t)N * sB, cudaMemcpyDeviceToHost, cs));
-  if (traj_y) CK(cudaMemcpyAsync(traj_y, d_ty, (size_t)N * sB, cudaMemcpyDeviceToHost, cs));
-  if (full) CK(cudaMemcpyAsync(full, d_full, (8 * (size_t)N - 2) * sB, cudaMemcpyDeviceToHost, cs));
-  if (status) CK(cudaMemcpyAsync(status, d_status, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, cs));
-  if (iters) CK(cudaMemcpyAsync(iters, d_iters, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, cs));
-  if (pre) {
+  cudaStream_t cs = pre.recorded ? h->stream2 : st;
+  if (pre.recorded) CK(cudaStreamWaitEvent(cs, h->ev_pre, 0));
+  CK(cudaMemcpyAsync(result, d.res, 9 * sB, cudaMemcpyDeviceToHost, cs));
+  if (traj_x) CK(cudaMemcpyAsync(traj_x, d.tx, (size_t)N * sB, cudaMemcpyDeviceToHost, cs));
+  if (traj_y) CK(cudaMemcpyAsync(traj_y, d.ty, (size_t)N * sB, cudaMemcpyDeviceToHost, cs));
+  if (full) CK(cudaMemcpyAsync(full, d.full, (8 * (size_t)N - 2) * sB, cudaMemcpyDeviceToHost, cs));
+  if (status) CK(cudaMemcpyAsync(status, d.status, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, cs));
+  if (iters) CK(cudaMemcpyAsync(iters, d.iters, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, cs));
+  if (pre.recorded) {
     CK(cudaEventRecord(h->ev_copy, cs));
     CK(cudaStreamWaitEvent(st, h->ev_copy, 0));
-    mpc_patch_outputs_kernel<<<h->sm_count, 256, 0, st>>>(h->pre_kp, h->pre_rec, h->pre_cki, pa);
+    mpc_patch_outputs_kernel<<<h->sm_count, 256, 0, st>>>(pre.kp, pre.rec, pre.cki, pa);
     CK(cudaGetLastError());
     h->launches++;
   }
@@ -1009,14 +1025,11 @@ extern "C" int mpc_solve_batch_multi(mpc_multi *m, int B, const double *state, c
     if (Bs == 0) return MPC_OK;
     mpc_handle *h = m->h[g];
     CK(cudaSetDevice(h->device));
-    int rc = ensure_staging(h, (size_t)Bs, N, weights != nullptr);
+    Staging d;
+    int rc = ensure_staging(h, (size_t)Bs, N, weights != nullptr, &d);
     if (rc) return rc;
     cudaStream_t st = h->stream;
-    const size_t cap = h->cap_B, w = (size_t)Bs * sizeof(double);
-    double *d_state = h->d_in, *d_coef = d_state + 6 * cap, *d_ylo = d_coef + 5 * cap, *d_yhi = d_ylo + cap;
-    double *d_w = d_yhi + cap, *d_dt = d_w + 12 * cap;
-    double *d_res = h->d_out, *d_tx = d_res + 9 * cap, *d_ty = d_tx + (size_t)N * cap, *d_full = d_ty + (size_t)N * cap;
-    int *d_status = h->d_iout, *d_iters = d_status + cap, *d_N = d_iters + cap;
+    const size_t w = (size_t)Bs * sizeof(double);
     // a shard of a [rows][B] array is `rows` runs of Bs values: one strided copy per array
     auto in2d = [&](double *dst, const double *src, int rows) {
       return cudaMemcpy2DAsync(dst, w, src + lo, pitchB, w, (size_t)rows, cudaMemcpyHostToDevice, st);
@@ -1024,30 +1037,29 @@ extern "C" int mpc_solve_batch_multi(mpc_multi *m, int B, const double *state, c
     auto out2d = [&](double *dst, const double *src, int rows) {
       return cudaMemcpy2DAsync(dst + lo, pitchB, src, w, w, (size_t)rows, cudaMemcpyDeviceToHost, st);
     };
-    CK(in2d(d_state, state, 6));
-    CK(in2d(d_coef, coeffs, 5));
-    CK(in2d(d_ylo, yaw_lo, 1));
-    CK(in2d(d_yhi, yaw_hi, 1));
-    if (weights) CK(in2d(d_w, weights, 12));
-    if (dt_per) CK(in2d(d_dt, dt_per, 1));
+    CK(in2d(d.state, state, 6));
+    CK(in2d(d.coef, coeffs, 5));
+    CK(in2d(d.ylo, yaw_lo, 1));
+    CK(in2d(d.yhi, yaw_hi, 1));
+    if (weights) CK(in2d(d.w, weights, 12));
+    if (dt_per) CK(in2d(d.dt, dt_per, 1));
     if (N_per) {
-      CK(cudaMemcpyAsync(d_N, N_per + lo, (size_t)Bs * sizeof(int), cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d.N, N_per + lo, (size_t)Bs * sizeof(int), cudaMemcpyHostToDevice, st));
       // rows at or beyond a problem's horizon stay as the caller left them (see mpc_solve_batch_host)
-      if (traj_x) CK(in2d(d_tx, traj_x, N));
-      if (traj_y) CK(in2d(d_ty, traj_y, N));
-      if (full) CK(in2d(d_full, full, 8 * N - 2));
+      if (traj_x) CK(in2d(d.tx, traj_x, N));
+      if (traj_y) CK(in2d(d.ty, traj_y, N));
+      if (full) CK(in2d(d.full, full, 8 * N - 2));
     }
-    h->want_pre = false;
-    rc = solve_batch(h, true, Bs, d_state, d_coef, d_ylo, d_yhi, weights ? d_w : nullptr, N_per ? d_N : nullptr,
-                         dt_per ? d_dt : nullptr, d_res, traj_x ? d_tx : nullptr, traj_y ? d_ty : nullptr,
-                         full ? d_full : nullptr, d_status, d_iters, st);
+    rc = solve_batch(h, bound_call(h, true), Bs, d.state, d.coef, d.ylo, d.yhi, weights ? d.w : nullptr,
+                     N_per ? d.N : nullptr, dt_per ? d.dt : nullptr, d.res, traj_x ? d.tx : nullptr,
+                     traj_y ? d.ty : nullptr, full ? d.full : nullptr, d.status, d.iters, st);
     if (rc) return rc;
-    CK(out2d(result, d_res, 9));
-    if (traj_x) CK(out2d(traj_x, d_tx, N));
-    if (traj_y) CK(out2d(traj_y, d_ty, N));
-    if (full) CK(out2d(full, d_full, 8 * N - 2));
-    if (status) CK(cudaMemcpyAsync(status + lo, d_status, (size_t)Bs * sizeof(int), cudaMemcpyDeviceToHost, st));
-    if (iters) CK(cudaMemcpyAsync(iters + lo, d_iters, (size_t)Bs * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(out2d(result, d.res, 9));
+    if (traj_x) CK(out2d(traj_x, d.tx, N));
+    if (traj_y) CK(out2d(traj_y, d.ty, N));
+    if (full) CK(out2d(full, d.full, 8 * N - 2));
+    if (status) CK(cudaMemcpyAsync(status + lo, d.status, (size_t)Bs * sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (iters) CK(cudaMemcpyAsync(iters + lo, d.iters, (size_t)Bs * sizeof(int), cudaMemcpyDeviceToHost, st));
     return MPC_OK;
   };
   int first_error = MPC_OK, queued = 0;
@@ -1077,7 +1089,7 @@ extern "C" int mpc_solve_one(mpc_handle *h, const double *state, const double *c
   if (!h || !state || !coeffs || !result) return MPC_EINVAL;
   CK(cudaSetDevice(h->device));
   const int N = h->cfg.N;
-  int rc = ensure_staging(h, 1, N, false);
+  int rc = ensure_staging(h, 1, N, false, nullptr);
   if (rc) return rc;
   cudaStream_t st = h->stream;
   double *hp = h->h_pin;                       // [13 inputs | 9 + 2N outputs | 2 ints]
@@ -1090,10 +1102,8 @@ extern "C" int mpc_solve_one(mpc_handle *h, const double *state, const double *c
   double *ho = hp + 16;
   int *hi = reinterpret_cast<int *>(hp + 16 + 9 + 2 * (size_t)N);
   double *full = nullptr;
-  bool warm = false;
-  const double *ws_save[4] = {h->ws_x, h->ws_lam, h->ws_zl, h->ws_zu};
-  double *dual_save[3] = {h->dual_lam, h->dual_zl, h->dual_zu};
-  const double ws_mu_save = h->ws_mu;
+  SolveCall call = bound_call(h, false);   // cold; the bound multiplier outputs unless the single-solve warm start is on
+  call.one_shot = true;
   if (h->one_warm) {
     // the last solution and the next start point, each [x 8N-2 | lambda 6N | zl 8N-2 | zu 8N-2] (B = 1): the solve
     // writes the first, the shift turns it into the second
@@ -1107,22 +1117,17 @@ extern "C" int mpc_solve_one(mpc_handle *h, const double *state, const double *c
     }
     double *sol = h->d_one, *nxt = h->d_one + per;
     full = sol;
-    h->dual_lam = sol + nx; h->dual_zl = sol + nx + 6 * N; h->dual_zu = sol + 2 * nx + 6 * N;
+    call.dual_lam = sol + nx; call.dual_zl = sol + nx + 6 * N; call.dual_zu = sol + 2 * nx + 6 * N;
     if (h->one_prev_ok) {
       rc = mpc_warm_start_shift(h, 1, sol, sol + nx, sol + nx + 6 * N, sol + 2 * nx + 6 * N, nxt, nxt + nx,
                                 nxt + nx + 6 * N, nxt + 2 * nx + 6 * N, st);
-      if (rc) { h->dual_lam = dual_save[0]; h->dual_zl = dual_save[1]; h->dual_zu = dual_save[2]; return rc; }
-      h->ws_x = nxt; h->ws_lam = nxt + nx; h->ws_zl = nxt + nx + 6 * N; h->ws_zu = nxt + 2 * nx + 6 * N;
-      h->ws_mu = h->one_mu > 0.0 ? h->one_mu : 0.1;
-      warm = true;
+      if (rc) return rc;
+      call.ws_x = nxt; call.ws_lam = nxt + nx; call.ws_zl = nxt + nx + 6 * N; call.ws_zu = nxt + 2 * nx + 6 * N;
+      call.ws_mu = h->one_mu > 0.0 ? h->one_mu : 0.1;
     }
   }
-  h->one_shot = true;
-  rc = solve_batch(h, warm, 1, hp, hp + 6, hp + 11, hp + 12, nullptr, nullptr, nullptr, ho, ho + 9, ho + 9 + N, full, hi,
+  rc = solve_batch(h, call, 1, hp, hp + 6, hp + 11, hp + 12, nullptr, nullptr, nullptr, ho, ho + 9, ho + 9 + N, full, hi,
                    hi + 1, st);
-  h->one_shot = false;
-  h->ws_x = ws_save[0]; h->ws_lam = ws_save[1]; h->ws_zl = ws_save[2]; h->ws_zu = ws_save[3]; h->ws_mu = ws_mu_save;
-  h->dual_lam = dual_save[0]; h->dual_zl = dual_save[1]; h->dual_zu = dual_save[2];
   if (rc) return rc;
   CK(cudaStreamSynchronize(st));
   if (h->one_warm) h->one_prev_ok = hi[0] == MPC_STATUS_SUCCESS;   // a failed solve is no start point
@@ -1270,8 +1275,8 @@ extern "C" int mpc_run_batch(mpc_handle *h, int B, const double *pose, const dou
   const int thr = 128, grid = (B + thr - 1) / thr;
   mpc_run_pre_kernel<<<grid, thr, 0, st>>>(h->cfg, R);
   CK(cudaGetLastError());
-  rc = solve_batch(h, false, B, R.state, R.coeffs, R.yaw_lo, R.yaw_hi, nullptr, nullptr, nullptr, result, traj_x, traj_y,
-                       nullptr, d_status, d_iters, st);
+  rc = solve_batch(h, bound_call(h, false), B, R.state, R.coeffs, R.yaw_lo, R.yaw_hi, nullptr, nullptr, nullptr, result,
+                   traj_x, traj_y, nullptr, d_status, d_iters, st);
   if (rc) return rc;
   mpc_run_post_kernel<<<grid, thr, 0, st>>>(h->cfg, B, R.aux, result, out8);
   CK(cudaGetLastError());
@@ -1282,29 +1287,12 @@ extern "C" int mpc_run_batch(mpc_handle *h, int B, const double *pose, const dou
 // the closed loop as one launch of mpc_rollout_kernel: a lane group per vehicle, all T steps
 template <int NS>
 static int launch_rollout(mpc_handle *h, const LoopArgs &A, int T, cudaStream_t st) {
-  const int threads = 128, G = NS <= 16 ? 16 : 32, groups = threads / G;
-  const size_t smem = (size_t)groups * NS * ST_ROW_SH * sizeof(double);
-  static thread_local int cached_dev = -1, per_sm = 0;
-  if (cached_dev != h->device) {
-    CK(cudaFuncSetAttribute(mpc_rollout_kernel<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mpc_rollout_kernel<NS>, threads, smem));
-    cached_dev = h->device;
-  }
-  if (per_sm < 1) { snprintf(g_err, sizeof(g_err), "rollout kernel does not fit on an SM (smem %zu)", smem); return MPC_ECUDA; }
-  long long want = ((long long)A.V + groups - 1) / groups, grid = (long long)h->sm_count * per_sm;
-  if (grid > want) grid = want;
-  if (grid < 1) grid = 1;
   KParams kp;
   fill_kparams(h->cfg, A.V, kp);
   kp.state = A.state; kp.coeffs = A.coeffs; kp.yaw_lo = A.yaw_lo; kp.yaw_hi = A.yaw_hi;
   kp.result = A.result; kp.status = const_cast<int *>(A.status); kp.iters = const_cast<int *>(A.iters);
   kp.handoff_iter = INT_MAX;
-  int rc = ensure_coop_scratch<NS>(h, kp, grid * groups);
-  if (rc) return rc;
-  mpc_rollout_kernel<NS><<<(unsigned)grid, threads, smem, st>>>(kp, h->cfg, A, T);
-  CK(cudaGetLastError());
-  h->launches++;
-  return MPC_OK;
+  return launch_coop_family<NS>(h, mpc_rollout_kernel<NS>, "rollout kernel", kp, A.V, st, h->cfg, A, T);
 }
 
 extern "C" int mpc_set_rollout_mode(mpc_handle *h, int mode) {
@@ -1335,22 +1323,14 @@ extern "C" int mpc_rollout(mpc_handle *h, int V, int T, const double *track_x, c
   const bool persistent = h->rollout_mode == MPC_ROLLOUT_PERSISTENT || (h->rollout_mode == MPC_ROLLOUT_AUTO && V <= MPC_ROLLOUT_PERSISTENT_MAX);
   if (persistent) {
     A.step = 0;
-    const int N = h->cfg.N;
-    if (N <= 10) return launch_rollout<10>(h, A, T, st);
-#ifndef MPC_DEV_N10
-    if (N <= 20) return launch_rollout<20>(h, A, T, st);
-    if (N <= 32) return launch_rollout<32>(h, A, T, st);
-    return launch_rollout<MPC_NMAX>(h, A, T, st);
-#else
-    return MPC_EINVAL;
-#endif
+    return with_horizon(h->cfg.N, [&](auto ns) { return launch_rollout<decltype(ns)::value>(h, A, T, st); });
   }
   const int thr = 128, grid = (V + thr - 1) / thr;
   for (int k = 0; k < T; k++) {
     A.step = k;
     mpc_loop_pre_kernel<<<grid, thr, 0, st>>>(h->cfg, A);
-    rc = solve_batch(h, false, V, A.state, A.coeffs, A.yaw_lo, A.yaw_hi, nullptr, nullptr, nullptr, A.result, nullptr,
-                         nullptr, nullptr, d_status, d_iters, st);
+    rc = solve_batch(h, bound_call(h, false), V, A.state, A.coeffs, A.yaw_lo, A.yaw_hi, nullptr, nullptr, nullptr,
+                     A.result, nullptr, nullptr, nullptr, d_status, d_iters, st);
     if (rc) return rc;
     mpc_loop_post_kernel<<<grid, thr, 0, st>>>(h->cfg, A);
     h->launches += 2;
@@ -1419,13 +1399,3 @@ extern "C" int mpc_tail_counts(mpc_handle *h, int *parked, int n) {
 extern "C" long long mpc_launch_count(const mpc_handle *h) { return h ? h->launches : 0; }
 extern "C" const char *mpc_last_error(void) { return g_err; }
 extern "C" const char *mpc_version(void) { return "mpc_b200 0.3 (sm_100a, fp64 interior point with restoration phase and watchdog; lane and coop kernels, explicit fma)"; }
-
-#ifdef MPC_DEBUG_TIMES
-// development builds only: per-warp "out of work" and exit times of the last main launch (tools/gpu_cta_times.py)
-extern "C" int mpc_debug_times(unsigned long long *out, int n, int reset) {
-  const int m = 4 + 148 * 9 * 2;
-  if (out && n >= m) CK(cudaMemcpyFromSymbol(out, mpcb200::g_dbg_times, m * sizeof(unsigned long long)));
-  if (reset) { static unsigned long long z[4 + 148 * 9 * 2]; CK(cudaMemcpyToSymbol(mpcb200::g_dbg_times, z, sizeof(z))); }
-  return MPC_OK;
-}
-#endif

@@ -90,37 +90,6 @@ enum { ST_S = 0,      // iterate: x, y, psi, v, cte, epsi
        ST_LH = 76,    // coop kernel only: StageLin (10) + StageHess (18) of the stage, built one stage per lane
        ST_ROW_SH = 106 };   // shared-memory rows: 104 used; 106 keeps neighbouring lanes' rows 2-way bank-conflict free
 template <int NS, bool SH, bool PAR> struct LaneRows { typedef double type[NS][ST_ROW]; enum { ROW = ST_ROW }; };
-// Experiment (profiles/r02_lane_rows_in_shared_memory.txt): some columns of the lane kernel's thread-private rows in
-// shared memory instead.  Two column ranges [A0, A1) and [B0, B1) (compile-time, -DMPC_LANE_SM_A0=.. etc.) map to NC slots;
-// slot k of stage i of thread t is at sm[(i * NC + k) * STRIDE + t] -- consecutive lanes, consecutive words, no bank
-// conflicts.  Column indices are compile-time constants after unrolling, so the choice costs no instruction.
-#ifndef MPC_LANE_SM_A0
-#define MPC_LANE_SM_A0 0
-#define MPC_LANE_SM_A1 0
-#define MPC_LANE_SM_B0 0
-#define MPC_LANE_SM_B1 0
-#endif
-#define MPC_LANE_SM_NC ((MPC_LANE_SM_A1 - MPC_LANE_SM_A0) + (MPC_LANE_SM_B1 - MPC_LANE_SM_B0))
-#define MPC_LANE_SM_STRIDE 224   /* threads per CTA of the lane kernel when the rows are hybrid */
-#define MPC_LANE_HYBRID(NS) (MPC_LANE_SM_NC > 0 && (NS) <= 10)
-template <int NS> struct HybridRows {
-  alignas(16) double loc[NS][ST_ROW];
-  double *sm;
-  struct Row {
-    double *l, *s;
-    __device__ __forceinline__ double &operator[](int c) const {
-      if (c >= MPC_LANE_SM_A0 && c < MPC_LANE_SM_A1) return s[(c - MPC_LANE_SM_A0) * MPC_LANE_SM_STRIDE];
-      if (c >= MPC_LANE_SM_B0 && c < MPC_LANE_SM_B1) return s[(c - MPC_LANE_SM_B0 + (MPC_LANE_SM_A1 - MPC_LANE_SM_A0)) * MPC_LANE_SM_STRIDE];
-      return l[c];
-    }
-  };
-  __device__ __forceinline__ Row operator[](int i) const {
-    return Row{const_cast<double *>(loc[i]), sm + (size_t)i * (MPC_LANE_SM_NC * MPC_LANE_SM_STRIDE)};
-  }
-};
-#if MPC_LANE_SM_NC > 0
-template <> struct LaneRows<10, false, false> { typedef HybridRows<10> type; enum { ROW = ST_ROW }; };
-#endif
 template <int NS> struct LaneRows<NS, true, true> { typedef double (*type)[ST_ROW_SH]; enum { ROW = ST_ROW_SH }; };
 template <int NS> struct LaneRows<NS, true, false> { typedef double (*type)[ST_ROW]; enum { ROW = ST_ROW }; };
 
@@ -3131,31 +3100,13 @@ __device__ __forceinline__ ChainIO chain_resolve(const KParams &P) {
 // RESUME = true is the same kernel started from the records of the previous launch instead of fresh problems,
 // 32 consecutive records to a warp, warps dealt round-robin to the CTAs -- so the survivors of many sparse
 // warps run in a few full ones.  The last launch of a chain parks nothing (P.ckpt == NULL).
-#ifdef MPC_DEBUG_TIMES
-// development aid (tools/gpu_cta_times.py): when does each warp of the main launch run out of work, when does its CTA exit
-__device__ unsigned long long g_dbg_times[4 + 148 * 9 * 2];
-__device__ __forceinline__ unsigned long long dbg_now() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-#endif
-template <int NS> __device__ __forceinline__ void lane_rows_attach(HybridRows<NS> &r, double *sm) { r.sm = sm; }
-template <class T> __device__ __forceinline__ void lane_rows_attach(T &, double *) {}
-#ifndef MPC_LANE_MAXT
-#define MPC_LANE_MAXT 256   // largest CTA the lane kernel is compiled for (register cap = 65536 / (MAXT * MINB)): experiments only
-#endif
+// The largest CTA the lane kernel is compiled for, one CTA per SM: a register budget of 65536 / 256 a thread
+// (profiles/r01_lane_threads_sweep.txt).
+enum { LANE_MAX_THREADS = 256 };
 // WARM: launches with a warm start (Lane::init); a resume launch may hold a warm problem parked before its first trip
-template <int NS, int MINB, bool RESUME, bool WARM>
-#ifdef MPC_LANE_MAXNREG
-__global__ void __maxnreg__(MPC_LANE_MAXNREG) mpc_lane_kernel(const KParams P) {
-#else
-__global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KParams P) {
-#endif
+template <int NS, bool RESUME, bool WARM>
+__global__ void __launch_bounds__(LANE_MAX_THREADS, 1) mpc_lane_kernel(const KParams P) {
   Lane<NS, false> Z;
-#if MPC_LANE_SM_NC > 0
-  extern __shared__ double lane_smem[];
-  if (MPC_LANE_HYBRID(NS)) lane_rows_attach(Z.ST, lane_smem + threadIdx.x);
-#endif
-#ifdef MPC_DEBUG_TIMES
-  if (!RESUME && threadIdx.x == 0) { if (blockIdx.x == 0) g_dbg_times[0] = dbg_now(); }
-#endif
   Z.mode = LM_IDLE;
   Z.b = 0;
   Z.g0 = 0; Z.gstep = 1; Z.gm = 0xffffffffu;
@@ -3209,13 +3160,6 @@ __global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KPa
         }
       }
     }
-#ifdef MPC_DEBUG_TIMES
-    if (!RESUME) {
-      const bool wdone = __all_sync(0xffffffffu, Z.mode == LM_DONE);
-      const int w = blockIdx.x * 9 + (threadIdx.x >> 5);
-      if (wdone && (threadIdx.x & 31) == 0 && g_dbg_times[4 + 2 * w] == 0) g_dbg_times[4 + 2 * w] = dbg_now();
-    }
-#endif
     if (__syncthreads_and(Z.mode == LM_DONE)) break;
     Z.trip_eval();
     Z.template trip_accept<WARM>(P);
@@ -3224,9 +3168,6 @@ __global__ void __launch_bounds__(MPC_LANE_MAXT, MINB) mpc_lane_kernel(const KPa
     // progress guard (see run_to_completion): a problem that stops making progress must not hold the whole grid
     if (Z.mode != LM_IDLE && Z.mode != LM_DONE && Z.mode != LM_FINISH && ++Z.trips > 64 * (P.max_iter + 16)) { Z.status = 13; Z.mode = LM_FINISH; }
   }
-#ifdef MPC_DEBUG_TIMES
-  if (!RESUME && (threadIdx.x & 31) == 0) g_dbg_times[4 + 2 * (blockIdx.x * 9 + (threadIdx.x >> 5)) + 1] = dbg_now();
-#endif
 }
 
 // The same solver with one problem per GROUP of 16 (N <= 16) or 32 lanes and the per-stage rows in shared
@@ -3268,10 +3209,7 @@ __global__ void __launch_bounds__(128, 2) mpc_coop_kernel(const KParams P) {
 // state and carries on from the trip where the lane stopped; then the problems that were handed over when no record
 // slot was free (restart_list) are solved from the start.
 template <int NS, bool WARM>
-#ifndef MPC_COOP_RESUME_MINB
-#define MPC_COOP_RESUME_MINB 2   // CTAs per SM the finisher is compiled for at N <= 10 (3 = 168 registers: experiment)
-#endif
-__global__ void __launch_bounds__(128, NS <= 10 ? MPC_COOP_RESUME_MINB : 2) mpc_coop_resume_kernel(const KParams P) {
+__global__ void __launch_bounds__(128, 2) mpc_coop_resume_kernel(const KParams P) {
   extern __shared__ double coop_smem[];
   const int G = Lane<NS, true>::NS_GROUP;
   const int lane = threadIdx.x & 31;

@@ -24,4 +24,4 @@ for thr, ctas in sets:
         e0.record(); S.solve_batch_device(B, state, coeffs, ylo, yhi, result, tx, ty, None, status, iters); e1.record()
         torch.cuda.synchronize()
         best = min(best, e0.elapsed_time(e1))
-    print('MINB=%s lane threads=%d ctas/sm=%d  B=%d  %.3f ms  %.0f solves/s  ok=%.4f iters=%.2f csum=%.6f' % (os.environ.get('MPC_LANE_MINB', '2'), thr, ctas, B, best, B / best * 1e3, (status == 1).float().mean().item(), iters.float().mean().item(), result[8].sum().item()))
+    print('lane threads=%d ctas/sm=%d  B=%d  %.3f ms  %.0f solves/s  ok=%.4f iters=%.2f csum=%.6f' % (thr, ctas, B, best, B / best * 1e3, (status == 1).float().mean().item(), iters.float().mean().item(), result[8].sum().item()))
