@@ -36,7 +36,7 @@ EXPORTS = ["mpc_config_defaults", "mpc_config_load_json", "mpc_config_parse_json
            "mpc_rollout", "mpc_set_handoff", "mpc_set_tail", "mpc_tail_counts", "mpc_measure_solve_latency", "mpc_set_dual_outputs", "mpc_config_from_cli",
            "mpc_telemetry_parse", "mpc_telemetry_step", "mpc_create_multi", "mpc_destroy_multi", "mpc_multi_device_count",
            "mpc_multi_handle", "mpc_solve_batch_multi", "mpc_set_rollout_mode", "mpc_set_warm_start", "mpc_warm_start_shift",
-           "mpc_set_warm_start_one"]
+           "mpc_set_warm_start_one", "mpc_solution_sensitivity"]
 
 
 class MpcError(RuntimeError):
@@ -129,6 +129,7 @@ def lib():
     L.mpc_set_warm_start.argtypes = [vp, vp, vp, vp, vp, C.c_double]
     L.mpc_set_warm_start_one.argtypes = [vp, C.c_int, C.c_double]
     L.mpc_warm_start_shift.argtypes = [vp, C.c_int] + [vp] * 8 + [vp]
+    L.mpc_solution_sensitivity.argtypes = [vp, C.c_int] + [vp] * 13 + [vp]
     L.mpc_telemetry_parse.argtypes = [C.c_char_p, C.POINTER(MpcTelemetry)]
     L.mpc_telemetry_step.argtypes = [vp, C.c_char_p, dp, C.c_double, C.c_int, C.c_char_p, C.c_int]
     L.mpc_solve_batch.argtypes = [vp, C.c_int] + [vp] * 13 + [vp]
@@ -393,6 +394,20 @@ class Solver:
             stream = torch.cuda.current_stream().cuda_stream
         _check(lib().mpc_warm_start_shift(self._h, int(B), _ptr(x), _ptr(lam), _ptr(zl), _ptr(zu), _ptr(x0), _ptr(lam0),
                                           _ptr(zl0), _ptr(zu0), stream), "mpc_warm_start_shift")
+
+    def solution_sensitivity(self, B, state, coeffs, yaw_lo, yaw_hi, full, lam, zl, zu, dresult, dfull=None, status=None,
+                             weights=None, dt_per=None, stream=None):
+        """Derivatives of solutions with respect to the initial state (mpc_solution_sensitivity): DEVICE tensors in the
+        [k][B] layout of solve_batch_device -- the problem arrays of the solve, its ``full``, the multipliers of
+        set_dual_outputs and (optionally) its status -> dresult [6][9][B] and dfull [6][8N-2][B] (or None), slice k =
+        d/d state_k.  Asynchronous on ``stream`` (None = torch's current stream)."""
+        if stream is None:
+            import torch
+            stream = torch.cuda.current_stream().cuda_stream
+        _check(lib().mpc_solution_sensitivity(self._h, int(B), _ptr(state), _ptr(coeffs), _ptr(yaw_lo), _ptr(yaw_hi),
+                                              _ptr(weights), _ptr(dt_per), _ptr(full), _ptr(lam), _ptr(zl), _ptr(zu),
+                                              _ptr(status), _ptr(dresult), _ptr(dfull), stream),
+               "mpc_solution_sensitivity")
 
     @property
     def launches(self):

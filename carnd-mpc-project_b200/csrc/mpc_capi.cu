@@ -22,6 +22,7 @@
 #include "mpc_kernel.cuh"
 #include "mpc_lane_kernel.cuh"
 #include "mpc_rollout.cuh"
+#include "mpc_sensitivity.cuh"
 #include "mpc_run_logic.h"
 
 using namespace mpcb200;
@@ -809,6 +810,27 @@ extern "C" int mpc_solve_batch(mpc_handle *h, int B, const double *state, const 
   if (!h) return MPC_EINVAL;
   return solve_batch(h, bound_call(h, true), B, state, coeffs, yaw_lo, yaw_hi, weights, N_per, dt_per, result, traj_x,
                      traj_y, full, status, iters, cuda_stream);
+}
+
+extern "C" int mpc_solution_sensitivity(mpc_handle *h, int B, const double *state, const double *coeffs,
+                                        const double *yaw_lo, const double *yaw_hi, const double *weights,
+                                        const double *dt_per, const double *full, const double *lambda, const double *zl,
+                                        const double *zu, const int *status, double *dresult, double *dfull,
+                                        void *cuda_stream) {
+  if (!h || B < 0 || !state || !coeffs || !yaw_lo || !yaw_hi || !full || !lambda || !zl || !zu || !dresult)
+    return MPC_EINVAL;
+  if (B == 0) return MPC_OK;
+  CK(cudaSetDevice(h->device));
+  KParams kp;
+  fill_kparams(h->cfg, B, kp);
+  kp.state = state; kp.coeffs = coeffs; kp.yaw_lo = yaw_lo; kp.yaw_hi = yaw_hi; kp.weights_pp = weights; kp.dt_pp = dt_per;
+  const SensArgs A = {full, lambda, zl, zu, status, dresult, dfull};
+  return with_horizon(h->cfg.N, [&](auto ns) {
+    mpc_sensitivity_kernel<decltype(ns)::value><<<(B + 127) / 128, 128, 0, (cudaStream_t)cuda_stream>>>(kp, A);
+    CK(cudaGetLastError());
+    h->launches++;
+    return MPC_OK;
+  });
 }
 
 // Early copy-back: the outputs of the problems the final launch of a chain finished, written again -- straight into

@@ -250,6 +250,25 @@ int mpc_set_warm_start(mpc_handle *h, const double *x0, const double *lambda0, c
 int mpc_warm_start_shift(mpc_handle *h, int B, const double *x, const double *lambda, const double *zl,
                          const double *zu, double *x0, double *lambda0, double *zl0, double *zu0, void *cuda_stream);
 
+/* Parametric sensitivity (Ipopt's sIPOPT) of solutions of mpc_solve_batch with respect to the initial state, for the
+ * UNSCALED problem at the given point.  DEVICE pointers on the handle's device, asynchronous on cuda_stream, one launch.
+ * Inputs: the problem arrays of the solve (state [6][B], coeffs [5][B], yaw_lo, yaw_hi [B], weights [12][B] or NULL,
+ *   dt_per [B] or NULL; per-problem horizons are not supported), the solution full [8*cfg.N-2][B] and the multipliers
+ *   lambda [6*cfg.N][B], zl, zu [8*cfg.N-2][B] in the layouts of mpc_set_dual_outputs, and status [B] or NULL.
+ * Outputs, slice k = derivative with respect to state component k (x, y, psi, v, cte, epsi):
+ *   dresult [6][9][B]            in the layout of `result` (x1..epsi1, delta0, a0, cost)
+ *   dfull   [6][8*cfg.N-2][B] or NULL, in the layout of `full`
+ * A problem whose status is neither MPC_STATUS_SUCCESS nor MPC_STATUS_STOP_AT_ACCEPTABLE_POINT (status NULL: every
+ * problem is computed), or whose reduced Hessian is not positive definite at the point, gets NaN in all its outputs.
+ * The derivative is that of the KKT system at the point, with the barrier term Sigma = zl / (z - lo) + zu / (hi - z) on
+ * the bounds relaxed as the solver relaxes them, and FG_eval's branches frozen at the problem's own state.  The cost
+ * row is grad f(z)^T dz, so it equals -lambda of the initial-condition row up to the barrier term and the solve's
+ * tolerance.  Independent of the handle's kernel choice, tail settings, warm start and dual outputs; changes none. */
+int mpc_solution_sensitivity(mpc_handle *h, int B, const double *state, const double *coeffs, const double *yaw_lo,
+                             const double *yaw_hi, const double *weights, const double *dt_per, const double *full,
+                             const double *lambda, const double *zl, const double *zu, const int *status,
+                             double *dresult, double *dfull, void *cuda_stream);
+
 /* One problem, host pointers: state[6], coeffs[5] -> result[9], traj_x/traj_y[N] (or NULL).
  * What `MPC::solve` calls once per telemetry message. */
 int mpc_solve_one(mpc_handle *h, const double *state, const double *coeffs,
